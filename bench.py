@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: primitive-loss forward+backward samples/s (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c1]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c3|c1] [--dump-outputs DIR]
 
 A step = one pass of the hot path over one synthetic batch: draw uniforms -> fused sample+pose of K
 primitives -> Chamfer NN (both directions) vs the targets (+ VP-diverse Chamfer, + mesh vertices ->
@@ -269,10 +269,12 @@ class Bench:
         return s
 
 
-def measure_workload(B, workload, steps, warmup, chamfer_impl=0, graph="auto", with_rooflines=True, cpu_baseline=False):
+def measure_workload(B, workload, steps, warmup, chamfer_impl=0, graph="auto", with_rooflines=True, cpu_baseline=False,
+                     keep_outputs=False):
     """value (device-resident inputs), e2e (pinned host inputs, copies inside the timed region) and, on rank 0, the
     rooflines of one workload.  Both timed regions run under the same conditions: 256 MB L2 flush before every step,
-    NVML clock sampling on rank 0, gradient all-reduce (N > 1) inside the step.  Returns a dict (rank 0) or None."""
+    NVML clock sampling on rank 0, gradient all-reduce (N > 1) inside the step.  Returns a dict (rank 0) or None.
+    keep_outputs: the result also holds, as numpy arrays under "outputs", what the last timed step returned."""
     vpn, dist, dev, world, rank, lib = B.vpn, B.dist, B.dev, B.world, B.rank, B.lib
     kind, b, k, n, m, res = WORKLOADS[workload]
     b = per_gpu_batch(workload, world)
@@ -280,6 +282,7 @@ def measure_workload(B, workload, steps, warmup, chamfer_impl=0, graph="auto", w
     faithful = workload in FAITHFUL
     width = 2 if kind == "sphere" else 3
     nsets = 4
+    torch.manual_seed(1234 + rank)            # the step's uniforms are drawn on the device: the same draws in every run
     host = synthetic(workload, "cpu", seed=1234 + rank, sets=nsets, batch=b)
     devsets = [{kk: (vv.to(dev) if vv is not None else None) for kk, vv in s.items()} for s in host]
     pinned = [{kk: (vv.pin_memory() if vv is not None else None) for kk, vv in s.items()} for s in host]
@@ -345,7 +348,7 @@ def measure_workload(B, workload, steps, warmup, chamfer_impl=0, graph="auto", w
         if B.do_flush:
             flush.zero_()                                           # L2 flush between timed iterations
         evs[i][0].record()
-        one_step(devsets[i % nsets])
+        last = one_step(devsets[i % nsets])
         mids[i].record()
         if sync is not None:
             sync.join()
@@ -358,6 +361,9 @@ def measure_workload(B, workload, steps, warmup, chamfer_impl=0, graph="auto", w
     sampler.stop()
     sampler.join(timeout=5.0)
     B.barrier()
+    # copied now: the graphed step returns static buffers, which the e2e loop below overwrites
+    outputs = ({name: x.detach().cpu().numpy() for name, x in zip(("loss", "grad_v", "grad_q", "grad_t"), last)}
+               if keep_outputs else None)
     step_ms = [a.elapsed_time(bb) for a, bb in evs]
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=dev)
     # per rank: mean step time and the part of it spent before the all-reduce's completion is awaited
@@ -432,6 +438,8 @@ def measure_workload(B, workload, steps, warmup, chamfer_impl=0, graph="auto", w
                                  "clock sampling on rank 0, all-reduce inside the step; one host synchronisation per step; "
                                  "vpn_b200.HostPipeline: the host-to-device copy of batch i + 1 overlaps step i, every "
                                  "batch and every result is copied every step"}}
+    if outputs is not None:
+        out["outputs"] = outputs
     if not with_rooflines:
         return out
 
@@ -579,8 +587,10 @@ def compact(r):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
-    ap.add_argument("--warmup", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline value (the JSON `value` and `ms_per_step`); the e2e loop times "
+                         "max(3, steps // 2) steps and each extra workload of --configs max(5, min(10, steps))")
+    ap.add_argument("--warmup", type=int, default=5, help="untimed steps before timing (at least 3)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -590,14 +600,27 @@ def main():
     ap.add_argument("--configs", default="auto",
                     help="extra workloads measured after the headline one and reported in the `configs` block of the same JSON "
                          "line: 'auto' = c3,c5,c2f,c4 when the headline is c2, 'none', or a comma-separated list")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the headline workload returned (loss and the gradients to "
+                         "v, q, t; rank 0) as DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to --impl ours")
         return run_reference(args)
     B = Bench(args)
     world, rank = B.world, B.rank
     warm = max(3, args.warmup)
     head = measure_workload(B, args.workload, args.steps, warm, args.chamfer_impl, args.graph, with_rooflines=True,
-                            cpu_baseline=(world == 1 and not args.no_cpu_baseline))
+                            cpu_baseline=(world == 1 and not args.no_cpu_baseline),
+                            keep_outputs=bool(args.dump_outputs))
+    if rank == 0 and args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in head.pop("outputs").items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     extras = []
     if args.configs == "auto":
         extras = ["c3", "c5", "c2f", "c4"] if args.workload == "c2" else []

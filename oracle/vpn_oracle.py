@@ -78,12 +78,33 @@ def rotation_matrices(qn: torch.Tensor) -> torch.Tensor:
     return torch.stack([r0, r1, r2], dim=1)
 
 
+def _fma(a: torch.Tensor, b: torch.Tensor, c: torch.Tensor) -> torch.Tensor:
+    """a * b + c rounded once to fp32: the product of two fp32 values is exact in fp64, and the fp64 sum rounds to the
+    same fp32 value as the exact sum unless it lands exactly halfway between two fp32 values."""
+    return (a.double() * b.double() + c.double()).float()
+
+
 def rotate_points(points: torch.Tensor, q: torch.Tensor) -> torch.Tensor:
-    """rotate.py:7-25.  out[b,n,:] = R(q[b]) @ points[b,n,:] (batched GEMM with k = 3)."""
+    """rotate.py:7-25.  out[b,n,:] = R(q[b]) @ points[b,n,:] (torch.bmm with k = 3).
+
+    torch.bmm's rounding depends on the host: below 400 multiply-adds per matrix ATen sums the products itself,
+    ((r0 x + r1 y) + r2 z) with every operation rounded; above, the CPU BLAS does, and whether its kernel fuses the
+    multiply-adds depends on the instruction set.  tests/golden/ was recorded where it evaluated
+    fma(r2, z, fma(r1, y, r0 x)).  Both orders are written out so that the oracle gives the same bits on every host,
+    except where _fma's fp64 sum lands exactly halfway between two fp32 values and rounds twice (rare).  With torch.bmm,
+    MKL_ENABLE_INSTRUCTIONS=AVX2 alone fails four golden tests of tests/test_oracle_golden.py."""
     assert points.ndimension() == 3 and points.size(-1) == 3      # rotate.py:49-51
     assert q.ndimension() == 2 and q.size(-1) == 4                # rotate.py:54-56
     mats = rotation_matrices(refine_quaternions(q))
-    return torch.bmm(mats, points.permute(0, 2, 1)).permute(0, 2, 1)
+    x, y, z = points[..., 0], points[..., 1], points[..., 2]
+    rows = []
+    for i in range(3):
+        r0, r1, r2 = (mats[:, i, j, None] for j in range(3))
+        if 9 * points.size(1) < 400:
+            rows.append((r0 * x + r1 * y) + r2 * z)
+        else:
+            rows.append(_fma(r2, z, _fma(r1, y, r0 * x)))
+    return torch.stack(rows, dim=2)
 
 
 def translate_points(points: torch.Tensor, t: torch.Tensor) -> torch.Tensor:

@@ -189,19 +189,14 @@ def test_clock_sampler_with_fake_nvml(monkeypatch):
 
 
 def test_reference_derived_test_binaries_build_here():
-    """oracle/_ref/ holds the two artefacts compiled from the reference's own code (EMD kernels -> libemd_ref.so, training
-    loop helpers -> train_helpers.bin).  They are built wherever /root/reference is mounted and shipped to the GPU box."""
+    """oracle/_ref/libemd_ref.so holds the reference's own EMD kernels, compiled from its source tree (VPN_REFERENCE_ROOT)
+    where that tree is at hand; nothing of the reference's text is tracked."""
     import subprocess
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("reference tree not mounted: the prebuilt binaries are used as shipped")
+    from oracle import ref_import
+    if not os.path.isfile(os.path.join(ref_import.REFERENCE_ROOT, "modules", "loss", "emd", "emd_cuda.cu")):
+        pytest.skip("the reference's source tree is not present")
     subprocess.check_call(["make", "-C", os.path.join(REPO, "oracle")])
     assert os.path.isfile(os.path.join(REPO, "oracle", "_ref", "libemd_ref.so"))
-    from oracle import build_ref_train_helpers as bld
-    names = {k: set(bld.load(k).co_names) for k in bld.CHUNKS}
-    assert {"sample_predict_points", "get_vp_meshes", "compose_vp_meshes", "calculate_cd_loss", "calculate_silhouette_loss",
-            "calculate_vp_div_loss", "calculate_emd_loss"} <= names["train"]
-    assert {"deform_meshes", "sample_points"} <= names["train_sphere"]
-    assert {"sample_predict_points", "get_vp_meshes", "compose_vp_meshes", "calculate_emd_loss"} <= names["train_gcn"]
     # nothing of the reference's text is tracked by git: _ref is ignored
     tracked = subprocess.run(["git", "-C", REPO, "ls-files", "oracle/_ref"], capture_output=True, text=True).stdout.strip()
     assert tracked == ""

@@ -1,10 +1,9 @@
-"""The reference's OWN training-loop helpers, executed unmodified against the drop-in `modules` package.
+"""The training scripts' loop helpers, restated, run against the drop-in `modules` package and compared with the CPU oracle.
 
-oracle/build_ref_train_helpers.py compiled train.py:105-195, train_sphere.py:62-80 and train_gcn.py:56-95 to bytecode
-(oracle/_ref/train_helpers.bin - a binary artefact, shipped to the GPU box; the reference tree itself is not).  Here
-those code objects are exec'd in a namespace that provides exactly what the scripts import (`from config import *`,
-`from modules.sampling import Sampling`, ...), but from THIS repository's drop-ins, and their results are compared with
-the CPU oracle.  This is the test behind INTEGRATION.md's "stays as written" column.
+The helpers of train.py:105-195, train_sphere.py:62-80 and train_gcn.py:56-95 call the hot-path modules in the order and
+with the arguments SURVEY.md section 3 records.  The scripts are not part of this repository, so `helpers()` restates
+those calls from that record, reading the same `config` constants, and every result and gradient is compared with the
+CPU oracle.  A call in the real scripts that differs from the record (another keyword or argument order) is not caught.
 """
 import os
 import sys
@@ -32,23 +31,67 @@ def O():
 
 
 def helpers(script, **overrides):
-    """Namespace of one reference script's helpers, bound to the drop-in modules (what the script's imports resolve to
-    when volumetric-primitives-net_b200/ is first on sys.path)."""
-    from oracle import build_ref_train_helpers as bld
-    assert os.path.isfile(bld.OUT), f"{bld.OUT} missing: run `make -C oracle` where /root/reference is mounted"
+    """Namespace of one training script's helpers, bound to the drop-in modules (what the script's imports resolve to
+    when volumetric-primitives-net_b200/ is first on sys.path); `overrides` replace config constants."""
     import config
     from modules.loss import ChamferDistanceLoss, EarthMoverDistanceLoss, SilhouetteLoss, VPDiverseLoss
-    from modules.meshing import Meshing, TriangleMesh
+    from modules.meshing import Meshing
     from modules.sampling import Sampling
-    from modules.transform import rotate_points_forward_x_axis, view_to_obj_points
-    ns = {k: getattr(config, k) for k in dir(config) if k.isupper()}
-    ns.update(torch=torch, Sampling=Sampling, Meshing=Meshing, TriangleMesh=TriangleMesh,
-              ChamferDistanceLoss=ChamferDistanceLoss, SilhouetteLoss=SilhouetteLoss, VPDiverseLoss=VPDiverseLoss,
-              EarthMoverDistanceLoss=EarthMoverDistanceLoss, view_to_obj_points=view_to_obj_points,
-              rotate_points_forward_x_axis=rotate_points_forward_x_axis)
-    ns.update(overrides)
-    exec(bld.load(script), ns)
-    return ns
+    from modules.transform import view_to_obj_points
+    c = {k: getattr(config, k) for k in dir(config) if k.isupper()}
+    c.update(overrides)
+    spheres_only = script == "train_gcn"                          # train_gcn.py: 16 spheres, hard-coded
+
+    def sample_predict_points(volumes, rotates, translates):      # train.py:105-120: per primitive, then cat
+        points = []
+        for i in range(len(volumes)):
+            cuboid = not spheres_only and i < c["CUBOID_NUM"]
+            sampling = Sampling.cuboid_sampling if cuboid else Sampling.sphere_sampling
+            points.append(sampling(volumes[i], rotates[i], translates[i], c["SAMPLE_NUM"]))
+        return torch.cat(points, dim=1)
+
+    def get_vp_meshes(volumes, rotates, translates):              # train.py:123-136: per primitive, B meshes each
+        meshes = []
+        for i in range(len(volumes)):
+            cuboid = not spheres_only and i < c["CUBOID_NUM"]
+            meshing = Meshing.cuboid_meshing if cuboid else Meshing.sphere_meshing
+            meshes.append(meshing(volumes[i], rotates[i], translates[i]))
+        return meshes
+
+    def compose_vp_meshes(vp_meshes):                             # train.py:139-149: one mesh per sample
+        return [Meshing.compose_meshes([m[b] for m in vp_meshes]) for b in range(len(vp_meshes[0]))]
+
+    def calculate_cd_loss(predict_points, canonical_points, view_center_points, dists, elevs, azims, angles):
+        # train.py:152-163: the canonical-frame term is computed even at its default weight L_CAN_CD = 0
+        predict_canonical = view_to_obj_points(predict_points, dists, elevs, azims, angles)
+        view_cd = ChamferDistanceLoss()(predict_points, view_center_points) * c["L_VIEW_CD"]
+        obj_cd = ChamferDistanceLoss()(predict_canonical, canonical_points) * c["L_CAN_CD"]
+        return view_cd, obj_cd
+
+    def calculate_silhouette_loss(predict_meshes, silhouettes, dists, elevs, azims):   # train.py:166-176
+        if c["L_SIL"] == 0:
+            return 0
+        if c["IS_VIEW_CENTER"]:                                   # the view-centred camera for every sample
+            dists, elevs, azims = torch.ones_like(dists), torch.zeros_like(elevs), torch.zeros_like(azims)
+        return SilhouetteLoss()(predict_meshes, silhouettes, dists, elevs, azims) * c["L_SIL"]
+
+    def calculate_vp_div_loss(translates, gt_points):             # train.py:179-185
+        return VPDiverseLoss()(translates, gt_points) * c["L_VP_DIV"]
+
+    def calculate_emd_loss(predict_points, gt_points):            # train.py:188-195, train_gcn.py:91-95
+        dist, _ = EarthMoverDistanceLoss()(predict_points, gt_points, 0.005, 50)
+        return torch.sqrt(dist).mean() * c["L_EMD"]
+
+    def deform_meshes(meshes, vertices_offset):                   # train_sphere.py:62-68
+        for b in range(len(meshes)):
+            meshes[b].vertices += vertices_offset[b]
+        return meshes
+
+    def sample_points(meshes):                                    # train_sphere.py:71-80
+        n = c["SAMPLE_NUM"] * (c["CUBOID_NUM"] + c["SPHERE_NUM"] + c["CONE_NUM"])
+        return torch.stack([m.sample(n)[0] for m in meshes])
+
+    return dict(locals())
 
 
 def prim_lists(O, b, k, seed, spread=0.3):
