@@ -151,6 +151,14 @@ int vpn_emd_fwd(const float* xyz1, const float* xyz2, float* dist, int* assignme
 /* grad_xyz1 (B,n,3) = 2 grad_dist (xyz1 - xyz2[assignment]); xyz2 receives no gradient (emd_module.py:66-67). */
 int vpn_emd_bwd(const float* xyz1, const float* xyz2, const int* assignment, const float* grad_dist,
                 float* grad_xyz1, int B, int n, void* stream);
+/* Fused loss head of train.py:188-195 / train_gcn.py:91-95: loss[b] = weight * mean_j sqrt(dist[b,j]) (IEEE sqrt), summed in an
+ * order that depends on n only, so a sample's value does not depend on the batch it is computed in.  The backward takes
+ * the per-sample upstream gradient grad_loss (B) and overwrites grad_xyz1 (B,n,3) in one pass, in the operation order of
+ * autograd through the head followed by vpn_emd_bwd (dist == 0 gives NaN, as in the reference). */
+int vpn_emd_loss_fwd(const float* dist, float weight, float* loss, float* scratch /* >= 32*B floats */, int B, int n,
+                     void* stream);
+int vpn_emd_loss_bwd(const float* xyz1, const float* xyz2, const int* assignment, const float* dist,
+                     const float* grad_loss, float weight, float* grad_xyz1, int B, int n, void* stream);
 
 /* ---- GCN vertex-feature pooling: modules/network/gcn.py:84-164 (train_gcn.py:121; SURVEY.md section 8f-4)
  * vpn_image_bounds: GCNModel.get_bound_of_images (gcn.py:90-133).  imgs (B,C,H,W) -> bounds (B,4) = [x lo, x hi, y lo,

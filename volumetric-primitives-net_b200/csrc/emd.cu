@@ -192,6 +192,61 @@ __global__ void emd_bwd_kernel(const float* __restrict__ xyz1, const float* __re
   gxyz1[3 * i] = g * (a[0] - t[0]); gxyz1[3 * i + 1] = g * (a[1] - t[1]); gxyz1[3 * i + 2] = g * (a[2] - t[2]);
 }
 
+// Loss head of train.py:188-195 / train_gcn.py:91-95, torch.sqrt(dist).mean() per sample: loss[b] = weight * (sum_j sqrt(dist[b,j]) / n).
+// Stage 1: kEmdLossSlices blocks per sample; block s sums the elements s * 256 + t + k * 256 * kEmdLossSlices in thread t,
+// then warps and blocks in a fixed tree.  Stage 2 adds the slices in index order.  The summation order depends on n only
+// (not on B, the auction's cluster size or the stream), so a sample's loss is the same bits in any batch.
+constexpr int kEmdLossSlices = 32;
+constexpr int kEmdLossThreads = 256;
+
+__global__ void __launch_bounds__(kEmdLossThreads)
+emd_loss_partial_kernel(const float* __restrict__ dist, float* __restrict__ partial, int n) {
+  __shared__ float red[kEmdLossThreads / 32];
+  const int b = blockIdx.x / kEmdLossSlices, sl = blockIdx.x % kEmdLossSlices;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const float* d = dist + (size_t)b * n;
+  float s = 0.f;
+  for (int j = sl * kEmdLossThreads + threadIdx.x; j < n; j += kEmdLossThreads * kEmdLossSlices) s = __fadd_rn(s, __fsqrt_rn(d[j]));
+  s = warp_sum(s);
+  if (lane == 0) red[warp] = s;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float a = 0.f;
+    for (int w = 0; w < kEmdLossThreads / 32; ++w) a += red[w];
+    partial[blockIdx.x] = a;
+  }
+}
+
+__global__ void emd_loss_final_kernel(const float* __restrict__ partial, float weight, float* __restrict__ loss, int B, int n) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  float a = 0.f;
+  for (int k = 0; k < kEmdLossSlices; ++k) a += partial[(size_t)b * kEmdLossSlices + k];
+  loss[b] = weight * (a / (float)n);
+}
+
+// Backward of the head and of the auction's dist in one pass, in autograd's operation order through
+// torch.sqrt(dist).mean(dim=1) * weight followed by NmDistanceGradKernel (emd_cuda.cu:283-300):
+//   g = (grad_loss[b] * weight) / n;  g = g / (2 sqrt(d));  grad_xyz1 = (2 g) (x1 - x2[assignment]).
+// d == 0 gives inf * 0 = NaN, as in the reference.
+__global__ void emd_loss_bwd_kernel(const float* __restrict__ xyz1, const float* __restrict__ xyz2,
+                                    const int* __restrict__ assignment, const float* __restrict__ dist,
+                                    const float* __restrict__ grad_loss, float weight, float* __restrict__ gxyz1,
+                                    size_t total, int n) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const size_t b = i / n;
+  const int k = assignment[i];
+  float g = __fdiv_rn(__fmul_rn(grad_loss[b], weight), (float)n);
+  g = __fdiv_rn(g, __fmul_rn(2.0f, __fsqrt_rn(dist[i])));
+  g = __fmul_rn(g, 2.0f);
+  const float* a = xyz1 + 3 * i;
+  const float* t = xyz2 + 3 * (b * n + (k < 0 ? 0 : k));
+  gxyz1[3 * i] = __fmul_rn(g, __fsub_rn(a[0], t[0]));
+  gxyz1[3 * i + 1] = __fmul_rn(g, __fsub_rn(a[1], t[1]));
+  gxyz1[3 * i + 2] = __fmul_rn(g, __fsub_rn(a[2], t[2]));
+}
+
 }  // namespace vpn
 
 using namespace vpn;
@@ -255,4 +310,28 @@ extern "C" int vpn_emd_bwd(const float* xyz1, const float* xyz2, const int* assi
   const size_t total = (size_t)B * n;
   emd_bwd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(xyz1, xyz2, assignment, grad_dist, grad_xyz1, total, n);
   return vpn_check_launch("emd_bwd_kernel");
+}
+
+// scratch: >= 32 * B floats of device memory (partial sums)
+extern "C" int vpn_emd_loss_fwd(const float* dist, float weight, float* loss, float* scratch, int B, int n, void* stream) {
+  if (B < 0 || n <= 0) { vpn_set_error("emd loss: bad shape B=%d n=%d", B, n); return VPN_ERR_SHAPE; }
+  if (B == 0) return VPN_OK;
+  if (!dist || !loss || !scratch) { vpn_set_error("emd loss: null pointer"); return VPN_ERR_ARG; }
+  cudaStream_t s = (cudaStream_t)stream;
+  emd_loss_partial_kernel<<<(unsigned)B * kEmdLossSlices, kEmdLossThreads, 0, s>>>(dist, scratch, n);
+  int rc = vpn_check_launch("emd_loss_partial_kernel");
+  if (rc) return rc;
+  emd_loss_final_kernel<<<(B + 127) / 128, 128, 0, s>>>(scratch, weight, loss, B, n);
+  return vpn_check_launch("emd_loss_final_kernel");
+}
+
+extern "C" int vpn_emd_loss_bwd(const float* xyz1, const float* xyz2, const int* assignment, const float* dist,
+                                const float* grad_loss, float weight, float* grad_xyz1, int B, int n, void* stream) {
+  if (B < 0 || n <= 0) { vpn_set_error("emd loss bwd: bad shape B=%d n=%d", B, n); return VPN_ERR_SHAPE; }
+  if (B == 0) return VPN_OK;
+  if (!xyz1 || !xyz2 || !assignment || !dist || !grad_loss || !grad_xyz1) { vpn_set_error("emd loss bwd: null pointer"); return VPN_ERR_ARG; }
+  const size_t total = (size_t)B * n;
+  emd_loss_bwd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(xyz1, xyz2, assignment, dist, grad_loss,
+                                                                                       weight, grad_xyz1, total, n);
+  return vpn_check_launch("emd_loss_bwd_kernel");
 }

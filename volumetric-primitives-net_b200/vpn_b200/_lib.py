@@ -52,6 +52,8 @@ _SIGNATURES = {
     "vpn_emd_workspace_bytes": (c_int, [c_int, c_int, POINTER(c_size_t)]),
     "vpn_emd_fwd": (c_int, [c_void_p] * 5 + [c_size_t, c_int, c_int, c_float, c_int, c_void_p]),
     "vpn_emd_bwd": (c_int, [c_void_p] * 5 + [c_int, c_int, c_void_p]),
+    "vpn_emd_loss_fwd": (c_int, [c_void_p, c_float, c_void_p, c_void_p, c_int, c_int, c_void_p]),
+    "vpn_emd_loss_bwd": (c_int, [c_void_p] * 5 + [c_float, c_void_p, c_int, c_int, c_void_p]),
     "vpn_image_bounds": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_float, c_void_p]),
     "vpn_points_yz_range": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "vpn_feature_pool_fwd": (c_int, [c_void_p] * 5 + [c_int] * 7 + [c_void_p]),

@@ -490,6 +490,52 @@ def emd_auction(xyz1, xyz2, eps: float, iters: int):
     return _EmdAuction.apply(xyz1, xyz2, eps, iters)
 
 
+class _EmdLoss(torch.autograd.Function):
+    """Per-sample loss weight * mean(sqrt(dist)) with the auction, the mean and the whole backward as vpn_b200 kernels
+    (no (B,n) gradient tensor, no elementwise torch launches)."""
+
+    @staticmethod
+    def forward(ctx, xyz1, xyz2, eps, iters, weight):
+        lib = _lib.load()
+        xyz1 = require(xyz1.contiguous(), f32, "xyz1"); xyz2 = require(xyz2.contiguous(), f32, "xyz2")
+        b, n, _ = xyz1.shape
+        dev = xyz1.device
+        dist = torch.empty((b, n), dtype=f32, device=dev)
+        assignment = torch.empty((b, n), dtype=torch.int32, device=dev)
+        nb = ctypes.c_size_t(0)
+        check(lib.vpn_emd_workspace_bytes(b, n, ctypes.byref(nb)), "vpn_emd_workspace_bytes")
+        ws = _scratch_bytes(nb.value, dev)
+        st = stream_ptr(dev)
+        check(lib.vpn_emd_fwd(ptr(xyz1), ptr(xyz2), ptr(dist), ptr(assignment), ptr(ws), nb.value, b, n, float(eps), int(iters),
+                              st), "vpn_emd_fwd")
+        loss = torch.empty((b,), dtype=f32, device=dev)
+        part = torch.empty((b * 32,), dtype=f32, device=dev)
+        check(lib.vpn_emd_loss_fwd(ptr(dist), float(weight), ptr(loss), ptr(part), b, n, st), "vpn_emd_loss_fwd")
+        ctx.save_for_backward(xyz1, xyz2, assignment, dist)
+        ctx.weight = float(weight)
+        return loss
+
+    @staticmethod
+    def backward(ctx, gloss):
+        lib = _lib.load()
+        xyz1, xyz2, assignment, dist = ctx.saved_tensors
+        b, n, _ = xyz1.shape
+        g1 = torch.empty_like(xyz1)
+        check(lib.vpn_emd_loss_bwd(ptr(xyz1), ptr(xyz2), ptr(assignment), ptr(dist), ptr(gloss.contiguous()), ctx.weight,
+                                   ptr(g1), b, n, stream_ptr(xyz1.device)), "vpn_emd_loss_bwd")
+        g2 = torch.zeros_like(xyz2) if ctx.needs_input_grad[1] else None      # emd_module.py:66-67: zeros for xyz2
+        return g1, g2, None, None, None
+
+
+def emd_distance(points1, points2, eps: float = 0.005, iters: int = 50, weight: float = 1.0, each_batch: bool = False):
+    """EMD loss term of train.py:188-195 / train_gcn.py:91-95, weight * torch.sqrt(dist).mean(), with the auction of
+    emd_auction (same preconditions: (B,n,3) clouds of equal shape, coordinates in [0,1]).  Returns the per-sample values
+    (B,) when each_batch, else their mean.  points2 receives a zero gradient, as in the reference."""
+    assert points1.dim() == 3 and points1.size(-1) == 3 and points2.shape == points1.shape     # emd_module.py:37-38
+    loss = _EmdLoss.apply(points1, points2, eps, iters, weight)
+    return loss if each_batch else loss.mean()
+
+
 def sample_primitives_ms(kind: str, v, q, t, uniform_sets, reps: int = 32) -> float:
     """Mean device time (ms) of one fused sample+pose launch over a stream of `reps` launches that rotate through
     `uniform_sets` (list of (B,K,N,2|3) tensors; make their total size exceed L2 for cold reads).  Measurement helper."""

@@ -1,5 +1,5 @@
-"""One primitive-loss step: the per-iteration primitive assembly + loss of train.py:243-258 (EMD excluded),
-batched over all K primitives and all B samples, every stage a vpn_b200 kernel.
+"""One primitive-loss step: the per-iteration primitive assembly + loss of train.py:243-260, batched over all K
+primitives and all B samples, every stage a vpn_b200 kernel.
 
     points   = sample + pose of K primitives            (train.py:105-120 -> one launch)
     view_cd  = Chamfer(points, view_center_points)       (train.py:152-163)
@@ -7,6 +7,7 @@ batched over all K primitives and all B samples, every stage a vpn_b200 kernel.
                                                           it even when its weight is 0, train.py:160-161)
     vp_div   = Chamfer(centres, targets, w1=.5, w2=1)    (train.py:179-185, vp_diverse.py:12-18)
     sil      = L1/MSE(soft_silhouette(mesh), gt)         (train.py:123-149,166-176; silhouette.py:13-23)
+    emd      = mean sqrt(auction dist)(points, targets)  (only when l_emd != 0; train.py:188-195, train_gcn.py:91-95)
 """
 from __future__ import annotations
 
@@ -33,6 +34,12 @@ class PrimitiveLossConfig:
     vertex_chamfer: bool = False      # train_gcn.py:127-130: the Chamfer term scores the composed mesh vertices, not samples
     soft_cull_backfaces: bool = False  # rasteriser soft pass: False = DIB-R (back faces culled by the coverage pass only)
     overlap_silhouette: bool = True   # run mesh -> silhouette -> image loss on a second stream, concurrently with the Chamfer terms
+    # EMD term (train.py:188-195, train_gcn.py:91-95).  The reference's config.py:17 sets L_EMD = 1.0; the default here is
+    # 0 so that every caller written before the term existed (bench.py's workloads among them) computes what it did.
+    # Pass l_emd=1.0 for the reference's training loss.  It needs as many points as targets (P == M).
+    l_emd: float = 0.0
+    emd_eps: float = 0.005            # train.py:188-195
+    emd_iters: int = 50
 
 
 class PrimitiveLoss:
@@ -70,6 +77,11 @@ class PrimitiveLoss:
         cfg = self.cfg
         out: Dict[str, torch.Tensor] = {}
         b, k = q.shape[:2]
+        if cfg.l_emd:
+            # the auction pairs every point with one target (emd_module.py:37-38): checked from the shapes before any launch
+            per_prim = templates.template(cfg.kind, v.device)[0].shape[0] if cfg.vertex_chamfer else uniforms.shape[2]
+            assert view_center_points.dim() == 3 and tuple(view_center_points.shape) == (b, k * per_prim, 3), (
+                f"l_emd needs as many points as targets: {k} x {per_prim} points, targets {tuple(view_center_points.shape)}")
         verts = None
         if cfg.vertex_chamfer:
             tv, _ = templates.template(cfg.kind, v.device)
@@ -104,6 +116,21 @@ class PrimitiveLoss:
                     sil_term.record_stream(cur); out["alpha"].record_stream(cur)
             else:
                 sil_term, out["alpha"] = self._silhouette_term(v, q, t, verts, silhouettes, sil_cameras)
+        # The EMD auction is one cluster launch that holds its SMs for milliseconds and shares nothing with the Chamfer
+        # terms but the points: forked like the silhouette branch, the other terms run on the SMs it leaves free.  Measured
+        # faster than running it inline on every workload of tools/bench_step_emd.py (DESIGN.md section 4.6).
+        emd_term, emd_side = None, None
+        if cfg.l_emd:
+            if self._fork_emd(points):
+                cur = torch.cuda.current_stream(v.device)
+                emd_side = self._side_stream(v.device, "emd")
+                emd_side.wait_stream(cur)
+                with torch.cuda.stream(emd_side):
+                    points.record_stream(emd_side)
+                    emd_term = self._emd_term(points, view_center_points)
+                    emd_term.record_stream(cur)
+            else:
+                emd_term = self._emd_term(points, view_center_points)
         if cfg.l_view_cd:
             add("view_cd", ops.chamfer_distance(points, view_center_points, w1=cfg.cd_w1, w2=cfg.cd_w2,
                                                 impl=cfg.chamfer_impl) * cfg.l_view_cd)
@@ -114,6 +141,10 @@ class PrimitiveLoss:
         if cfg.l_vp_div:
             add("vp_div", ops.chamfer_distance(t.contiguous(), view_center_points, w1=0.5, w2=1.0,
                                                impl=cfg.chamfer_impl) * cfg.l_vp_div)
+        if emd_term is not None:
+            if emd_side is not None:
+                torch.cuda.current_stream(v.device).wait_stream(emd_side)
+            add("emd", emd_term)
         if sil_term is not None:
             if side is not None:
                 torch.cuda.current_stream(v.device).wait_stream(side)
@@ -121,12 +152,23 @@ class PrimitiveLoss:
         out["total"] = total
         return out
 
-    def _side_stream(self, device):
-        key = ("side", str(device))
+    def _side_stream(self, device, name="side"):
+        key = (name, str(device))
         cache = self.__dict__.setdefault("_streams", {})
         if key not in cache:
             cache[key] = torch.cuda.Stream(device=device)
         return cache[key]
+
+    def _fork_emd(self, points) -> bool:
+        """Run the EMD term on its own stream whenever another term can use the SMs the auction leaves free
+        (tools/bench_step_emd.py overrides this to time both placements)."""
+        cfg = self.cfg
+        return points.is_cuda and bool(cfg.l_view_cd or cfg.l_can_cd or cfg.l_vp_div or cfg.l_sil)
+
+    def _emd_term(self, points, targets):
+        """l_emd * mean over the batch of mean sqrt(dist) (train.py:188-195; train_gcn.py:91-95)."""
+        cfg = self.cfg
+        return ops.emd_distance(points, targets, eps=cfg.emd_eps, iters=cfg.emd_iters, weight=cfg.l_emd)
 
     def _silhouette_term(self, v, q, t, verts, silhouettes, sil_cameras):
         """l_sil * L1|MSE(soft alpha, gt) and alpha (train.py:123-149,166-176; silhouette.py:13-23)."""
