@@ -140,6 +140,16 @@ int vpn_mesh_sample_fwd(const float* verts, const int* faces, const float* u, fl
                         float* cdf, int B, int V, int F, int n, void* stream);
 int vpn_mesh_sample_bwd(const int* faces, const float* u, const int* face_idx, const float* grad_points,
                         float* grad_verts, int B, int V, int F, int n, void* stream);
+/* The same gradient as a gather with a fixed summation order (what the autograd Function uses): the samples of each mesh
+ * are stably counting-sorted by face, each face sums w * grad over its run, each vertex sums its incident (face, corner)
+ * terms in CSR order.  No atomics and no memset; a mesh's grad_verts is the same bits in every run and in any batch.
+ * adj_offsets (V+1) int32 / adj_entries (3F) int32: vertex -> (3 * face + corner) CSR of `faces`, entries of a vertex in
+ * the order the caller chooses (vpn_b200: a stable argsort of faces.flatten()).  face_idx as vpn_mesh_sample_fwd wrote
+ * it.  workspace: vpn_mesh_sample_bwd_workspace_bytes(B, F, n) bytes of scratch. */
+int vpn_mesh_sample_bwd_workspace_bytes(int B, int F, int n, size_t* bytes);
+int vpn_mesh_sample_bwd_sorted(const int* faces, const float* u, const int* face_idx, const float* grad_points,
+                               float* grad_verts, const int* adj_offsets, const int* adj_entries, void* workspace,
+                               size_t workspace_bytes, int B, int V, int F, int n, void* stream);
 
 /* ---- EMD approximation by auction: modules/loss/emd (emd_module.py:29-79, emd_cuda.cu:227-316)
  * xyz1 (B,n,3) predicted (bidders), xyz2 (B,n,3) ground truth (objects), coordinates normalised to [0,1].

@@ -49,6 +49,8 @@ _SIGNATURES = {
                            + [c_size_t] + [c_int] * 5 + [c_void_p]),
     "vpn_mesh_sample_fwd": (c_int, [c_void_p] * 6 + [c_int] * 4 + [c_void_p]),
     "vpn_mesh_sample_bwd": (c_int, [c_void_p] * 5 + [c_int] * 4 + [c_void_p]),
+    "vpn_mesh_sample_bwd_workspace_bytes": (c_int, [c_int, c_int, c_int, POINTER(c_size_t)]),
+    "vpn_mesh_sample_bwd_sorted": (c_int, [c_void_p] * 8 + [c_size_t] + [c_int] * 4 + [c_void_p]),
     "vpn_emd_workspace_bytes": (c_int, [c_int, c_int, POINTER(c_size_t)]),
     "vpn_emd_fwd": (c_int, [c_void_p] * 5 + [c_size_t, c_int, c_int, c_float, c_int, c_void_p]),
     "vpn_emd_bwd": (c_int, [c_void_p] * 5 + [c_int, c_int, c_void_p]),

@@ -396,7 +396,7 @@ def _check_face_indices(faces: torch.Tensor, n_verts: int):
     key = (faces.data_ptr(), tuple(faces.shape), faces._version, int(n_verts), str(faces.device))
     if key in _FACES_CHECKED:
         return
-    if torch.cuda.is_current_stream_capturing():
+    if faces.is_cuda and torch.cuda.is_current_stream_capturing():
         return                                   # cannot read back while capturing; the eager warm-up call has checked
     if faces.numel():
         lo, hi = int(faces.min()), int(faces.max())
@@ -435,10 +435,38 @@ class _MeshSample(torch.autograd.Function):
         faces, u, face_idx = ctx.saved_tensors
         b, v, f, n = ctx.dims
         dev = u.device
+        offsets, entries = mesh_adjacency(faces, v)
         gverts = torch.empty((b, v, 3), dtype=f32, device=dev)
-        check(lib.vpn_mesh_sample_bwd(ptr(faces), ptr(u), ptr(face_idx), ptr(gpoints.contiguous()), ptr(gverts), b, v, f, n,
-                                      stream_ptr(dev)), "vpn_mesh_sample_bwd")
+        nb = ctypes.c_size_t(0)
+        check(lib.vpn_mesh_sample_bwd_workspace_bytes(b, f, n, ctypes.byref(nb)), "vpn_mesh_sample_bwd_workspace_bytes")
+        ws = _scratch_bytes(nb.value, dev)
+        check(lib.vpn_mesh_sample_bwd_sorted(ptr(faces), ptr(u), ptr(face_idx), ptr(gpoints.contiguous()), ptr(gverts),
+                                             ptr(offsets), ptr(entries), ptr(ws), nb.value, b, v, f, n, stream_ptr(dev)),
+              "vpn_mesh_sample_bwd_sorted")
         return gverts, None, None
+
+
+_ADJACENCY = {}
+
+
+def mesh_adjacency(faces: torch.Tensor, n_verts: int):
+    """Vertex -> (face, corner) CSR of a faces tensor (F,3) int32: (offsets (V+1,) int32, entries (3F,) int32 = 3 * face +
+    corner), a vertex's entries in increasing order.  It fixes the order in which the sampler's backward sums a vertex's
+    gradient.  Built on the device with torch, without a host read, and cached once per faces tensor outside graph
+    capture; the cache holds the tensor, so its storage cannot be reused under a cached key."""
+    key = (faces.data_ptr(), tuple(faces.shape), faces._version, int(n_verts), str(faces.device))
+    hit = _ADJACENCY.get(key)
+    if hit is not None:
+        return hit[1], hit[2]
+    flat = faces.reshape(-1).long()
+    entries = torch.argsort(flat, stable=True)
+    offsets = torch.searchsorted(flat[entries], torch.arange(n_verts + 1, device=faces.device))
+    if torch.cuda.is_current_stream_capturing():
+        return offsets.int(), entries.int()          # filled in only when the graph replays: not for eager callers
+    if len(_ADJACENCY) >= 64:
+        _ADJACENCY.clear()
+    _ADJACENCY[key] = (faces, offsets.int(), entries.int())
+    return _ADJACENCY[key][1], _ADJACENCY[key][2]
 
 
 def sample_mesh_surface(verts, faces, uniforms):

@@ -42,7 +42,98 @@ class PrimitiveLossConfig:
     emd_iters: int = 50
 
 
-class PrimitiveLoss:
+class _LossStep:
+    """What the batched steps share: the view-centred silhouette cameras, the side streams their independent branches are
+    forked onto, and the EMD term.  Subclasses have a `cfg` with l_emd / emd_eps / emd_iters and say whether they compute
+    any other term (_has_other_terms)."""
+
+    def default_cameras(self, b: int, device):
+        """IS_VIEW_CENTER cameras: dist = 1, elev = azim = 0 for every sample (train.py:172-174); built once per batch size."""
+        key = ("cam", b, str(device))
+        cache = self.__dict__.setdefault("_cams", {})
+        if key not in cache:
+            cache[key] = ops.look_at_cameras(torch.zeros(b, device=device), torch.zeros(b, device=device),
+                                             torch.ones(b, device=device))
+        return cache[key]
+
+    def _side_stream(self, device, name="side"):
+        key = (name, str(device))
+        cache = self.__dict__.setdefault("_streams", {})
+        if key not in cache:
+            cache[key] = torch.cuda.Stream(device=device)
+        return cache[key]
+
+    def _forked(self, device, name, fn, uses=()):
+        """fn() -> tuple of tensors, run on side stream `name` after the work queued so far on the caller's stream.
+        `uses`: tensors made by the step that the branch reads.  Returns (outputs, side stream); pass the stream to _join
+        before the outputs are used on the caller's stream.  Autograd runs the branch's backward on the same side stream;
+        under CUDA-graph capture the fork / join becomes two parallel branches of the graph."""
+        cur = torch.cuda.current_stream(device)
+        side = self._side_stream(device, name)
+        side.wait_stream(cur)
+        with torch.cuda.stream(side):
+            for x in uses:
+                x.record_stream(side)
+            outs = fn()
+            for o in outs:
+                o.record_stream(cur)
+        return outs, side
+
+    @staticmethod
+    def _join(device, side):
+        if side is not None:
+            torch.cuda.current_stream(device).wait_stream(side)
+
+    def _has_other_terms(self) -> bool:
+        raise NotImplementedError
+
+    def _fork_emd(self, points) -> bool:
+        """Run the EMD term on its own stream whenever another term can use the SMs the auction leaves free
+        (tools/bench_step_emd.py overrides this to time both placements)."""
+        return points.is_cuda and self._has_other_terms()
+
+    def _emd_term(self, points, targets):
+        """l_emd * mean over the batch of mean sqrt(dist) (train.py:188-195; train_gcn.py:91-95)."""
+        cfg = self.cfg
+        return ops.emd_distance(points, targets, eps=cfg.emd_eps, iters=cfg.emd_iters, weight=cfg.l_emd)
+
+    def _emd_branch(self, points, targets):
+        """(EMD term, its side stream or None).  The auction is one cluster launch that holds its SMs for milliseconds and
+        shares nothing with the other terms but the points: forked, the other terms run on the SMs it leaves free.
+        Measured faster than running it inline on every workload of tools/bench_step_emd.py (DESIGN.md section 4.6)."""
+        if self._fork_emd(points):
+            (term,), side = self._forked(points.device, "emd", lambda: (self._emd_term(points, targets),), uses=(points,))
+            return term, side
+        return self._emd_term(points, targets), None
+
+
+def _image_loss(alpha, silhouettes, kind: str, weight: float):
+    """weight * L1Loss | MSELoss of the soft alpha (B,H,W) against the ground truth (B,1,H,W) (silhouette.py:13-23)."""
+    diff = alpha[:, None] - silhouettes
+    sil = diff.abs().mean() if kind == "L1" else (diff * diff).mean()
+    return sil * weight
+
+
+def _capture(run, device, warmup: int):
+    """Run `run` `warmup` times on a side stream (caches, function attributes, allocator), then capture one call into a
+    CUDA graph.  Returns (graph, what the captured call returned, our kernel launches in one replay)."""
+    from . import _lib
+    side = torch.cuda.Stream(device=device)
+    side.wait_stream(torch.cuda.current_stream(device))
+    with torch.cuda.stream(side):
+        for _ in range(warmup):
+            run()
+    torch.cuda.current_stream(device).wait_stream(side)
+    torch.cuda.synchronize(device)
+    lib = _lib.load()
+    n0 = lib.vpn_launch_count()
+    graph = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(graph):
+        outs = run()
+    return graph, outs, int(lib.vpn_launch_count() - n0)
+
+
+class PrimitiveLoss(_LossStep):
     def __init__(self, config: Optional[PrimitiveLossConfig] = None):
         self.cfg = config or PrimitiveLossConfig()
         assert self.cfg.kind in ("sphere", "cuboid")
@@ -55,15 +146,6 @@ class PrimitiveLoss:
             tv, tf = templates.template(self.cfg.kind, device)
             nv = tv.shape[0]
             cache[key] = torch.cat([tf + i * nv for i in range(k)], dim=0).contiguous()
-        return cache[key]
-
-    def default_cameras(self, b: int, device):
-        """IS_VIEW_CENTER cameras: dist = 1, elev = azim = 0 for every sample (train.py:172-174); built once per batch size."""
-        key = ("cam", b, str(device))
-        cache = self.__dict__.setdefault("_cams", {})
-        if key not in cache:
-            cache[key] = ops.look_at_cameras(torch.zeros(b, device=device), torch.zeros(b, device=device),
-                                             torch.ones(b, device=device))
         return cache[key]
 
     def __call__(self, v: torch.Tensor, q: torch.Tensor, t: torch.Tensor, uniforms: torch.Tensor,
@@ -107,30 +189,14 @@ class PrimitiveLoss:
             if sil_cameras is None:
                 self.default_cameras(b, v.device)          # cached constants are created on the caller's stream, before the fork
             self.composed_faces(k, v.device)
+            sil = lambda: self._silhouette_term(v, q, t, verts, silhouettes, sil_cameras)
             if fork:
-                cur = torch.cuda.current_stream(v.device)
-                side = self._side_stream(v.device)
-                side.wait_stream(cur)
-                with torch.cuda.stream(side):
-                    sil_term, out["alpha"] = self._silhouette_term(v, q, t, verts, silhouettes, sil_cameras)
-                    sil_term.record_stream(cur); out["alpha"].record_stream(cur)
+                (sil_term, out["alpha"]), side = self._forked(v.device, "side", sil)
             else:
-                sil_term, out["alpha"] = self._silhouette_term(v, q, t, verts, silhouettes, sil_cameras)
-        # The EMD auction is one cluster launch that holds its SMs for milliseconds and shares nothing with the Chamfer
-        # terms but the points: forked like the silhouette branch, the other terms run on the SMs it leaves free.  Measured
-        # faster than running it inline on every workload of tools/bench_step_emd.py (DESIGN.md section 4.6).
+                sil_term, out["alpha"] = sil()
         emd_term, emd_side = None, None
         if cfg.l_emd:
-            if self._fork_emd(points):
-                cur = torch.cuda.current_stream(v.device)
-                emd_side = self._side_stream(v.device, "emd")
-                emd_side.wait_stream(cur)
-                with torch.cuda.stream(emd_side):
-                    points.record_stream(emd_side)
-                    emd_term = self._emd_term(points, view_center_points)
-                    emd_term.record_stream(cur)
-            else:
-                emd_term = self._emd_term(points, view_center_points)
+            emd_term, emd_side = self._emd_branch(points, view_center_points)
         if cfg.l_view_cd:
             add("view_cd", ops.chamfer_distance(points, view_center_points, w1=cfg.cd_w1, w2=cfg.cd_w2,
                                                 impl=cfg.chamfer_impl) * cfg.l_view_cd)
@@ -142,33 +208,17 @@ class PrimitiveLoss:
             add("vp_div", ops.chamfer_distance(t.contiguous(), view_center_points, w1=0.5, w2=1.0,
                                                impl=cfg.chamfer_impl) * cfg.l_vp_div)
         if emd_term is not None:
-            if emd_side is not None:
-                torch.cuda.current_stream(v.device).wait_stream(emd_side)
+            self._join(v.device, emd_side)
             add("emd", emd_term)
         if sil_term is not None:
-            if side is not None:
-                torch.cuda.current_stream(v.device).wait_stream(side)
+            self._join(v.device, side)
             add("sil", sil_term)
         out["total"] = total
         return out
 
-    def _side_stream(self, device, name="side"):
-        key = (name, str(device))
-        cache = self.__dict__.setdefault("_streams", {})
-        if key not in cache:
-            cache[key] = torch.cuda.Stream(device=device)
-        return cache[key]
-
-    def _fork_emd(self, points) -> bool:
-        """Run the EMD term on its own stream whenever another term can use the SMs the auction leaves free
-        (tools/bench_step_emd.py overrides this to time both placements)."""
+    def _has_other_terms(self) -> bool:
         cfg = self.cfg
-        return points.is_cuda and bool(cfg.l_view_cd or cfg.l_can_cd or cfg.l_vp_div or cfg.l_sil)
-
-    def _emd_term(self, points, targets):
-        """l_emd * mean over the batch of mean sqrt(dist) (train.py:188-195; train_gcn.py:91-95)."""
-        cfg = self.cfg
-        return ops.emd_distance(points, targets, eps=cfg.emd_eps, iters=cfg.emd_iters, weight=cfg.l_emd)
+        return bool(cfg.l_view_cd or cfg.l_can_cd or cfg.l_vp_div or cfg.l_sil)
 
     def _silhouette_term(self, v, q, t, verts, silhouettes, sil_cameras):
         """l_sil * L1|MSE(soft alpha, gt) and alpha (train.py:123-149,166-176; silhouette.py:13-23)."""
@@ -185,9 +235,7 @@ class PrimitiveLoss:
             sd, se, sa = sil_cameras
             rot, pos = ops.look_at_cameras(sa, se, sd)
         alpha, _, _ = ops.soft_silhouette(verts, faces, rot, pos, h, w, soft_cull_backfaces=cfg.soft_cull_backfaces)
-        diff = alpha[:, None] - silhouettes
-        sil = diff.abs().mean() if cfg.silhouette_loss == "L1" else (diff * diff).mean()
-        return sil * cfg.l_sil, alpha
+        return _image_loss(alpha, silhouettes, cfg.silhouette_loss, cfg.l_sil), alpha
 
 
 class GraphedPrimitiveLoss:
@@ -208,7 +256,6 @@ class GraphedPrimitiveLoss:
         e.g. GradientAllReduce.launch(inline=True) when the all-reduce is our own self-synchronising kernel, so that no
         host launch sits between the step's tail and the collective.  It also runs in each of the `warmup` eager steps
         (every rank makes the same number of calls)."""
-        from . import _lib
         self.cfg = config
         self.step = PrimitiveLoss(config)
         dev = v.device
@@ -234,19 +281,7 @@ class GraphedPrimitiveLoss:
                 after_backward()
             return out["total"], gv, gq, gt
 
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        with torch.cuda.stream(side):                      # warm-up off the capture: caches, function attributes, allocator
-            for _ in range(warmup):
-                run()
-        torch.cuda.current_stream(dev).wait_stream(side)
-        torch.cuda.synchronize(dev)
-        lib = _lib.load()
-        n0 = lib.vpn_launch_count()
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
-            self.loss, self.gv, self.gq, self.gt = run()
-        self.launches_per_step = int(lib.vpn_launch_count() - n0)      # our kernels inside one replay
+        self.graph, (self.loss, self.gv, self.gq, self.gt), self.launches_per_step = _capture(run, dev, warmup)
 
     def __call__(self, v, q, t, targets, silhouettes=None, canonical_points=None, cameras=None):
         if self.canonical is not None and canonical_points is not None:
@@ -262,6 +297,147 @@ class GraphedPrimitiveLoss:
             self.sil.copy_(silhouettes, non_blocking=True)
         self.graph.replay()
         return self.loss, self.gv, self.gq, self.gt
+
+
+@dataclass
+class MeshLossConfig:
+    """Loss of the two loops whose free variable is a mesh's vertex tensor (one topology for the whole batch):
+    train_sphere.py (n_samples > 0: area-weighted surface samples of the deformed sphere, train_sphere.py:71-80) and
+    train_gcn.py (n_samples = 0: the predicted vertices themselves)."""
+    n_samples: int = 2048             # train_sphere.py: SAMPLE_NUM * VP_NUM = 128 * 16 per mesh; 0 = score the vertices
+    l_cd: float = 1.0                 # config.py:14 (L_VIEW_CD)
+    cd_w1: float = 1.0                # config.py:12-13
+    cd_w2: float = 1.0
+    l_sil: float = 0.0                # config.py:16; silhouette of the mesh from the view-centred camera (train_sphere.py:125-128)
+    silhouette_loss: str = "L1"       # config.py:27
+    # EMD term: off by default for the reason given at PrimitiveLossConfig.l_emd; train_gcn.py adds it with weight 1.
+    # It needs as many points (n_samples, or V) as targets.
+    l_emd: float = 0.0
+    emd_eps: float = 0.005
+    emd_iters: int = 50
+    chamfer_impl: int = ops.CHAMFER_AUTO
+    soft_cull_backfaces: bool = False
+
+
+class MeshLoss(_LossStep):
+    """One loss step on a batch of meshes, every stage a vpn_b200 kernel; the gradient goes to `verts`.
+
+        points = verts                                      (n_samples == 0: train_gcn.py)
+               | area-weighted samples of the surface       (n_samples > 0: train_sphere.py, TriangleMesh.sample)
+        cd     = Chamfer(points, targets, cd_w1, cd_w2)
+        sil    = L1/MSE(soft_silhouette(verts, faces), gt)  (only when l_sil != 0; own stream when cd is on)
+        emd    = mean sqrt(auction dist)(points, targets)   (only when l_emd != 0; own stream when another term is on)
+
+    train_sphere.py passes verts = template + offsets (the offsets' gradient is the vertices'); train_gcn.py passes the
+    network's vertices.  The branches are placed on streams as in PrimitiveLoss."""
+
+    def __init__(self, config: Optional[MeshLossConfig] = None):
+        self.cfg = config or MeshLossConfig()
+        assert self.cfg.n_samples >= 0
+
+    def _has_other_terms(self) -> bool:
+        return bool(self.cfg.l_cd or self.cfg.l_sil)
+
+    def __call__(self, verts: torch.Tensor, faces: torch.Tensor, targets: torch.Tensor, uniforms: Optional[torch.Tensor] = None,
+                 silhouettes: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+        """verts (B,V,3), faces (F,3) int32, targets (B,M,3); uniforms (B,n_samples,3) in [0,1) = [face draw, u1, u2],
+        drawn on the device when None; silhouettes (B,1,H,W) when l_sil != 0.  Every check below reads shapes only, so
+        a failing call raises AssertionError before any launch (and the checks are safe under graph capture)."""
+        cfg = self.cfg
+        n = cfg.n_samples
+        assert verts.dim() == 3 and verts.size(-1) == 3, "verts must be (B, V, 3)"
+        assert faces.dim() == 2 and faces.size(-1) == 3, "faces must be (F, 3)"
+        b, nv = verts.shape[:2]
+        assert n > 0 or uniforms is None, "n_samples = 0 scores the vertices: uniforms have nothing to draw"
+        assert uniforms is None or tuple(uniforms.shape) == (b, n, 3), (
+            f"uniforms must be (B, n_samples, 3) = {(b, n, 3)}, got {tuple(uniforms.shape)}")
+        if cfg.l_emd:
+            # the auction pairs every point with one target (emd_module.py:37-38)
+            assert targets.dim() == 3 and tuple(targets.shape) == (b, n or nv, 3), (
+                f"l_emd needs as many points as targets: {n or nv} points per mesh, targets {tuple(targets.shape)}")
+        assert not cfg.l_sil or silhouettes is not None, "l_sil needs the ground-truth silhouettes"
+        ops._check_face_indices(faces, nv)
+        out: Dict[str, torch.Tensor] = {}
+        if n:
+            if uniforms is None:
+                uniforms = torch.rand((b, n, 3), device=verts.device)       # drawn on the device, as TriangleMesh.sample_batch does
+            points = ops.sample_mesh_surface(verts, faces, uniforms)[0]
+        else:
+            points = verts
+        out["points"] = points
+        total = None
+
+        def add(name, val):
+            nonlocal total
+            out[name] = val
+            total = val if total is None else total + val
+
+        sil_term, side = None, None
+        if cfg.l_sil:
+            self.default_cameras(b, verts.device)            # cached constants are created on the caller's stream, before the fork
+            sil = lambda: self._silhouette_term(verts, faces, silhouettes)
+            if verts.is_cuda and cfg.l_cd:
+                (sil_term, out["alpha"]), side = self._forked(verts.device, "side", sil)
+            else:
+                sil_term, out["alpha"] = sil()
+        emd_term, emd_side = None, None
+        if cfg.l_emd:
+            emd_term, emd_side = self._emd_branch(points, targets)
+        if cfg.l_cd:
+            add("cd", ops.chamfer_distance(points, targets, w1=cfg.cd_w1, w2=cfg.cd_w2, impl=cfg.chamfer_impl) * cfg.l_cd)
+        if emd_term is not None:
+            self._join(verts.device, emd_side)
+            add("emd", emd_term)
+        if sil_term is not None:
+            self._join(verts.device, side)
+            add("sil", sil_term)
+        out["total"] = total
+        return out
+
+    def _silhouette_term(self, verts, faces, silhouettes):
+        cfg = self.cfg
+        rot, pos = self.default_cameras(verts.size(0), verts.device)
+        h, w = silhouettes.shape[-2:]
+        alpha, _, _ = ops.soft_silhouette(verts, faces, rot, pos, h, w, soft_cull_backfaces=cfg.soft_cull_backfaces)
+        return _image_loss(alpha, silhouettes, cfg.silhouette_loss, cfg.l_sil), alpha
+
+
+class GraphedMeshLoss:
+    """MeshLoss - draw the uniforms, forward, backward to the vertices - captured once into a CUDA graph and replayed,
+    as GraphedPrimitiveLoss does for the primitive step.  The topology is fixed at construction; vertices, targets and
+    silhouettes are copied into static buffers, results are read from static buffers.
+
+        g = GraphedMeshLoss(cfg, verts, faces, targets, silhouettes)   # example tensors give the shapes
+        loss, grad_verts = g(verts, targets, silhouettes)             # overwritten by the next call
+        offsets.backward(grad_verts)                                  # train_sphere.py: verts = template + offsets
+    """
+
+    def __init__(self, config: MeshLossConfig, verts, faces, targets, silhouettes=None, warmup: int = 3):
+        self.cfg = config
+        self.step = MeshLoss(config)
+        dev = verts.device
+        self.verts = verts.detach().clone().requires_grad_()
+        self.faces = faces.detach().clone()
+        self.targets = targets.detach().clone()
+        self.sil = None if silhouettes is None else silhouettes.detach().clone()
+
+        def run():
+            out = self.step(self.verts, self.faces, self.targets, silhouettes=self.sil)
+            (gv,) = torch.autograd.grad(out["total"], (self.verts,))
+            return out["total"], gv
+
+        # the sampler's backward reads the cached vertex CSR of these faces: build it before the capture and keep it
+        # alive as long as the graph
+        self._adjacency = ops.mesh_adjacency(self.faces, verts.size(1)) if config.n_samples and verts.is_cuda else None
+        self.graph, (self.loss, self.gv), self.launches_per_step = _capture(run, dev, warmup)
+
+    def __call__(self, verts, targets, silhouettes=None):
+        self.verts.data.copy_(verts, non_blocking=True)
+        self.targets.copy_(targets, non_blocking=True)
+        if self.sil is not None and silhouettes is not None:
+            self.sil.copy_(silhouettes, non_blocking=True)
+        self.graph.replay()
+        return self.loss, self.gv
 
 
 class HostPipeline:
