@@ -69,6 +69,22 @@ int vpn_pose_bwd_workspace_floats(int nprim, int N, size_t* floats);
 int vpn_pose_points_bwd(int kind, const float* v, const float* q, const float* src, const float* grad_out,
                         float* grad_v, float* grad_q, float* grad_t, float* grad_points,
                         float* workspace, size_t workspace_floats, int nprim, int N, void* stream);
+/* Mixed cuboid + sphere assemblies (train.py's CUBOID_NUM cuboids followed by SPHERE_NUM spheres): primitive b*K + k is
+ * a cuboid when k < Kc, else a sphere; one forward launch and one backward pair for all B*K primitives.
+ * mode 0 = sampled (src_c = uniforms (B,Kc,N,3), src_s = uniforms (B,K-Kc,N,2), Nc = Ns = N)
+ * mode 1 = template (src_c = cuboid template (Nc,3), src_s = sphere template (Ns,3))
+ * v,q,t (B*K, 3|4|3), t may be NULL; out (B, Kc*Nc + (K-Kc)*Ns, 3): primitive (b,k)'s rows start at
+ * b*(Kc*Nc + (K-Kc)*Ns) + (k < Kc ? k*Nc : Kc*Nc + (k-Kc)*Ns).  A primitive's points, and its gradients for the same
+ * slice of grad_out, are the bits vpn_pose_points_fwd / _bwd give for its kind.  A kind without primitives may pass a
+ * NULL source.  Bad counts (B, K, Nc, Ns <= 0, Kc outside [0, K], Nc != Ns in mode 0) return VPN_ERR_SHAPE; a bad
+ * mode or a NULL pointer VPN_ERR_ARG; a short workspace VPN_ERR_WORKSPACE - all before any CUDA call. */
+int vpn_pose_mixed_fwd(int mode, const float* v, const float* q, const float* t, const float* src_c,
+                       const float* src_s, float* out, int B, int K, int Kc, int Nc, int Ns, void* stream);
+int vpn_pose_mixed_bwd_workspace_floats(int B, int K, int Kc, int Nc, int Ns, size_t* floats);
+/* grad_out (B, Kc*Nc + (K-Kc)*Ns, 3) -> grad_v (B*K,3), grad_q (B*K,4), grad_t (B*K,3); any may be NULL. */
+int vpn_pose_mixed_bwd(int mode, const float* v, const float* q, const float* src_c, const float* src_s,
+                       const float* grad_out, float* grad_v, float* grad_q, float* grad_t, float* workspace,
+                       size_t workspace_floats, int B, int K, int Kc, int Nc, int Ns, void* stream);
 /* get_faces_points (modules/sampling/cuboid.py:30-53): counts (nprim,6) int32. */
 int vpn_cuboid_face_counts(const float* v, int* counts, int nprim, int N, void* stream);
 

@@ -113,25 +113,25 @@ __device__ __forceinline__ void rotate_add(const PrimShared& ps, const float* c,
   o[2] = __fadd_rn(fmaf(r[8], c[2], fmaf(r[7], c[1], r[6] * c[0])), ps.t[2]);
 }
 
-// grid: x = primitive (b*K + k), y = slice of kPoseThreads * kPosePointsPerThread * kPoseSteps points.
+// One CTA's slice of one primitive: points [y * 2048, y * 2048 + 2048) of the primitive's N, y = blockIdx.y.  Its source
+// rows are those of primitive src_prim of src (all of src for the shared template), its output rows those of primitive
+// out_prim of out; its pose (v, q, t) is primitive prim's.
 // All source loads of the CTA are issued before the pose (sin, cos, sqrt, divisions by one thread) is waited for.
-// Launched as a programmatic dependent launch: the launch latency overlaps the tail of the previous kernel.
 template <int KIND>
-__global__ void __launch_bounds__(kPoseThreads)
-pose_fwd_kernel(const float* __restrict__ v, const float* __restrict__ q, const float* __restrict__ t,
-                const float* __restrict__ src, float* __restrict__ out, int N, int vec_ok) {
+__device__ __forceinline__ void pose_fwd_body(PrimShared& ps, const float* __restrict__ v, const float* __restrict__ q,
+                                              const float* __restrict__ t, const float* __restrict__ src, size_t src_prim,
+                                              float* __restrict__ out, size_t out_prim, size_t prim, int N, int vec_ok,
+                                              unsigned tid) {
   constexpr int W = SrcWidth<KIND>::value;
-  __shared__ PrimShared ps;
-  const size_t prim = blockIdx.x;
-  const int base_n = blockIdx.y * (kPoseThreads * kPosePointsPerThread * kPoseSteps) + threadIdx.x * kPosePointsPerThread;
+  const int base_n = blockIdx.y * (kPoseThreads * kPosePointsPerThread * kPoseSteps) + tid * kPosePointsPerThread;
   pdl_enter();      // launched with launch_pdl: this CTA may already be resident while the previous kernel drains
   float u[kPoseSteps][4 * W];
 #pragma unroll
   for (int s = 0; s < kPoseSteps; ++s) {
     const int n0 = base_n + s * kPoseThreads * kPosePointsPerThread;
-    if (n0 < N) load_src4<KIND>(src, prim, n0, N, vec_ok, u[s]);
+    if (n0 < N) load_src4<KIND>(src, src_prim, n0, N, vec_ok, u[s]);
   }
-  if (threadIdx.x == 0) load_prim(KIND, ps, v, q, t, (int)prim, N);
+  if (tid == 0) load_prim(KIND, ps, v, q, t, (int)prim, N);
   __syncthreads();
 #pragma unroll
   for (int s = 0; s < kPoseSteps; ++s) {
@@ -148,7 +148,7 @@ pose_fwd_kernel(const float* __restrict__ v, const float* __restrict__ q, const 
         rotate_add(ps, c, o[i]);
       }
     }
-    float* dst = out + 3 * (prim * (size_t)N + n0);
+    float* dst = out + 3 * (out_prim * (size_t)N + n0);
     if (vec_ok && cnt == kPosePointsPerThread) {
       float4* d4 = reinterpret_cast<float4*>(dst);
       d4[0] = make_float4(o[0][0], o[0][1], o[0][2], o[1][0]);
@@ -160,21 +160,76 @@ pose_fwd_kernel(const float* __restrict__ v, const float* __restrict__ q, const 
   }
 }
 
+// grid: x = primitive (b*K + k), y = slice of kPoseThreads * kPosePointsPerThread * kPoseSteps points.
+// Launched as a programmatic dependent launch: the launch latency overlaps the tail of the previous kernel.
+template <int KIND>
+__global__ void __launch_bounds__(kPoseThreads)
+pose_fwd_kernel(const float* __restrict__ v, const float* __restrict__ q, const float* __restrict__ t,
+                const float* __restrict__ src, float* __restrict__ out, int N, int vec_ok) {
+  __shared__ PrimShared ps;
+  const size_t prim = blockIdx.x;
+  pose_fwd_body<KIND>(ps, v, q, t, src, prim, out, prim, prim, N, vec_ok, threadIdx.x);
+}
+
+// A mixed assembly: primitive k of every sample is a cuboid when k < Kc, else a sphere (train.py's order).
+// Output row of the first point of primitive (b, k): b * (Kc*Nc + (K-Kc)*Ns) + (k < Kc ? k*Nc : Kc*Nc + (k-Kc)*Ns).
+struct MixedPrim {
+  bool cuboid;
+  int N;
+  size_t row;       // first output row
+  size_t src_prim;  // index of the primitive among those of its kind (b*Kc + k or b*(K-Kc) + k-Kc)
+};
+
+__device__ __forceinline__ MixedPrim mixed_prim(int prim, int K, int Kc, int Nc, int Ns) {
+  const int b = prim / K, k = prim - b * K, Ks = K - Kc;
+  MixedPrim m;
+  m.cuboid = k < Kc;
+  m.N = m.cuboid ? Nc : Ns;
+  m.row = (size_t)b * ((size_t)Kc * Nc + (size_t)Ks * Ns) + (m.cuboid ? (size_t)k * Nc : (size_t)Kc * Nc + (size_t)(k - Kc) * Ns);
+  m.src_prim = m.cuboid ? (size_t)b * Kc + k : (size_t)b * Ks + (k - Kc);
+  return m;
+}
+
+// One launch over all B*K primitives of a mixed assembly.  The kind is uniform across a CTA, which runs the same body
+// as pose_fwd_kernel<kind> on the same source rows: the primitive's points are the bits the single-kind kernel writes.
+// TEMPLATE: src_c / src_s are the cuboid / sphere templates; otherwise the (B,Kc,N,3) / (B,K-Kc,N,2) uniforms.
+// grid.y covers the larger kind; CTAs past the end of a primitive's slices return.
+template <bool TEMPLATE>
+__global__ void __launch_bounds__(kPoseThreads)
+pose_mixed_fwd_kernel(const float* __restrict__ v, const float* __restrict__ q, const float* __restrict__ t,
+                      const float* __restrict__ src_c, const float* __restrict__ src_s, float* __restrict__ out,
+                      int K, int Kc, int Nc, int Ns, int vec_ok) {
+  __shared__ PrimShared ps;
+  const int prim = blockIdx.x;
+  const MixedPrim m = mixed_prim(prim, K, Kc, Nc, Ns);
+  if ((int)blockIdx.y * (kPoseThreads * kPosePointsPerThread * kPoseSteps) >= m.N) return;     // before any memory access
+  float* dst = out + 3 * m.row;
+  if (TEMPLATE) {
+    pose_fwd_body<KIND_TEMPLATE>(ps, v, q, t, m.cuboid ? src_c : src_s, 0, dst, 0, prim, m.N, vec_ok, threadIdx.x);
+  } else if (m.cuboid) {
+    pose_fwd_body<KIND_CUBOID>(ps, v, q, t, src_c, m.src_prim, dst, 0, prim, m.N, vec_ok, threadIdx.x);
+  } else {
+    pose_fwd_body<KIND_SPHERE>(ps, v, q, t, src_s, m.src_prim, dst, 0, prim, m.N, vec_ok, threadIdx.x);
+  }
+}
+
 // Backward, stage 1: per block partial sums of
 //   [0..8]  G = sum_n g_n (x) c_n      (dL/dR)
 //   [9..11] sum_n g_n                  (dL/dt)
 //   [12..14] sum_n (R^T g_n) (.) d_n   (dL/dv)
+// over one CTA's slice y = blockIdx.y of one primitive, written to slot prim * gridDim.y + y of `partial` (16 floats
+// a slot).  Its source rows are those of primitive src_prim of src, its gradient rows (gout, and gpts) those of
+// primitive g_prim.
 // KIND_POINTS also writes dL/dpoints = R^T g.
 template <int KIND>
-__global__ void __launch_bounds__(kPoseThreads, 3)
-pose_bwd_partial_kernel(const float* __restrict__ v, const float* __restrict__ q,
-                        const float* __restrict__ src, const float* __restrict__ gout,
-                        float* __restrict__ partial, float* __restrict__ gpts, int N, int vec_ok) {
+__device__ __forceinline__ void pose_bwd_partial_body(PrimShared& ps, float (&red)[kPoseThreads / 32][16],
+                                                      const float* __restrict__ v, const float* __restrict__ q,
+                                                      const float* __restrict__ src, size_t src_prim,
+                                                      const float* __restrict__ gout, size_t g_prim,
+                                                      float* __restrict__ partial, float* __restrict__ gpts, size_t prim,
+                                                      int N, int vec_ok, unsigned tid) {
   constexpr int W = SrcWidth<KIND>::value;
-  __shared__ PrimShared ps;
-  __shared__ float red[kPoseThreads / 32][16];
-  const size_t prim = blockIdx.x;
-  const int base_n = blockIdx.y * (kPoseThreads * kPosePointsPerThread * kPoseSteps) + threadIdx.x * kPosePointsPerThread;
+  const int base_n = blockIdx.y * (kPoseThreads * kPosePointsPerThread * kPoseSteps) + tid * kPosePointsPerThread;
   float acc[15];
 #pragma unroll
   for (int i = 0; i < 15; ++i) acc[i] = 0.f;
@@ -183,9 +238,9 @@ pose_bwd_partial_kernel(const float* __restrict__ v, const float* __restrict__ q
 #pragma unroll
   for (int s = 0; s < 2; ++s) {
     const int n0 = base_n + s * kPoseThreads * kPosePointsPerThread;
-    if (n0 < N) { load_src4<KIND>(src, prim, n0, N, vec_ok, u[s]); load_src4<KIND_POINTS>(gout, prim, n0, N, vec_ok, gg[s]); }
+    if (n0 < N) { load_src4<KIND>(src, src_prim, n0, N, vec_ok, u[s]); load_src4<KIND_POINTS>(gout, g_prim, n0, N, vec_ok, gg[s]); }
   }
-  if (threadIdx.x == 0) load_prim(KIND, ps, v, q, nullptr, (int)prim, N);
+  if (tid == 0) load_prim(KIND, ps, v, q, nullptr, (int)prim, N);
   __syncthreads();
   const float* r = ps.pose.r;
 #pragma unroll
@@ -212,7 +267,7 @@ pose_bwd_partial_kernel(const float* __restrict__ v, const float* __restrict__ q
 #pragma unroll
           for (int a = 0; a < 3; ++a) acc[12 + a] += rg[a] * d[a];
           if (KIND == KIND_POINTS && gpts) {
-            float* o = gpts + 3 * (prim * (size_t)N + n);
+            float* o = gpts + 3 * (g_prim * (size_t)N + n);
             o[0] = rg[0]; o[1] = rg[1]; o[2] = rg[2];
           }
         }
@@ -220,22 +275,71 @@ pose_bwd_partial_kernel(const float* __restrict__ v, const float* __restrict__ q
     }
     if (s + 2 < kPoseSteps) {
       const int n2 = base_n + (s + 2) * kPoseThreads * kPosePointsPerThread;
-      if (n2 < N) { load_src4<KIND>(src, prim, n2, N, vec_ok, u[s & 1]); load_src4<KIND_POINTS>(gout, prim, n2, N, vec_ok, gg[s & 1]); }
+      if (n2 < N) { load_src4<KIND>(src, src_prim, n2, N, vec_ok, u[s & 1]); load_src4<KIND_POINTS>(gout, g_prim, n2, N, vec_ok, gg[s & 1]); }
     }
   }
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int lane = tid & 31, warp = tid >> 5;
 #pragma unroll
   for (int i = 0; i < 15; ++i) {
     float s = warp_sum(acc[i]);
     if (lane == 0) red[warp][i] = s;
   }
   __syncthreads();
-  if (threadIdx.x < 15) {
+  if (tid < 15) {
     float s = 0.f;
 #pragma unroll
-    for (int w = 0; w < kPoseThreads / 32; ++w) s += red[w][threadIdx.x];
-    partial[(prim * gridDim.y + blockIdx.y) * 16 + threadIdx.x] = s;
+    for (int w = 0; w < kPoseThreads / 32; ++w) s += red[w][tid];
+    partial[(prim * gridDim.y + blockIdx.y) * 16 + tid] = s;
   }
+}
+
+// partial: slot (prim * gridDim.y + slice) of 16 floats.
+template <int KIND>
+__global__ void __launch_bounds__(kPoseThreads, 3)
+pose_bwd_partial_kernel(const float* __restrict__ v, const float* __restrict__ q,
+                        const float* __restrict__ src, const float* __restrict__ gout,
+                        float* __restrict__ partial, float* __restrict__ gpts, int N, int vec_ok) {
+  __shared__ PrimShared ps;
+  __shared__ float red[kPoseThreads / 32][16];
+  const size_t prim = blockIdx.x;
+  pose_bwd_partial_body<KIND>(ps, red, v, q, src, prim, gout, prim, partial, gpts, prim, N, vec_ok, threadIdx.x);
+}
+
+// Mixed assembly (see pose_mixed_fwd_kernel): each CTA runs pose_bwd_partial_kernel<kind>'s body on its primitive's
+// rows and slice, so slot (prim * gridDim.y + slice) holds the bits the single-kind kernel writes for that slice.
+// Slots past a primitive's slices_for(N of its kind) are neither written nor read.  Two CTAs per SM instead of three:
+// the cuboid and sphere bodies in one kernel need more than the 80 registers that three allow.
+template <bool TEMPLATE>
+__global__ void __launch_bounds__(kPoseThreads, 2)
+pose_mixed_bwd_partial_kernel(const float* __restrict__ v, const float* __restrict__ q, const float* __restrict__ src_c,
+                              const float* __restrict__ src_s, const float* __restrict__ gout, float* __restrict__ partial,
+                              int K, int Kc, int Nc, int Ns, int vec_ok) {
+  __shared__ PrimShared ps;
+  __shared__ float red[kPoseThreads / 32][16];
+  const int prim = blockIdx.x;
+  const MixedPrim m = mixed_prim(prim, K, Kc, Nc, Ns);
+  if ((int)blockIdx.y * (kPoseThreads * kPosePointsPerThread * kPoseSteps) >= m.N) return;
+  const float* g = gout + 3 * m.row;
+  if (TEMPLATE) {
+    pose_bwd_partial_body<KIND_TEMPLATE>(ps, red, v, q, m.cuboid ? src_c : src_s, 0, g, 0, partial, nullptr, prim, m.N, vec_ok, threadIdx.x);
+  } else if (m.cuboid) {
+    pose_bwd_partial_body<KIND_CUBOID>(ps, red, v, q, src_c, m.src_prim, g, 0, partial, nullptr, prim, m.N, vec_ok, threadIdx.x);
+  } else {
+    pose_bwd_partial_body<KIND_SPHERE>(ps, red, v, q, src_s, m.src_prim, g, 0, partial, nullptr, prim, m.N, vec_ok, threadIdx.x);
+  }
+}
+
+// Backward, stage 2 tail for one primitive: acc = its summed slots; chains dL/dR to dL/dq and stores the gradients.
+__device__ __forceinline__ void pose_bwd_chain(const float* __restrict__ q, const float (&acc)[15], int prim,
+                                               float* __restrict__ gv, float* __restrict__ gq, float* __restrict__ gt) {
+  if (gq) {
+    Pose pose; make_pose(q + 4 * (size_t)prim, pose);
+    float g4[4]; pose_backward(q + 4 * (size_t)prim, pose, acc, g4);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) gq[4 * (size_t)prim + i] = g4[i];
+  }
+  if (gt) { gt[3 * (size_t)prim] = acc[9]; gt[3 * (size_t)prim + 1] = acc[10]; gt[3 * (size_t)prim + 2] = acc[11]; }
+  if (gv) { gv[3 * (size_t)prim] = acc[12]; gv[3 * (size_t)prim + 1] = acc[13]; gv[3 * (size_t)prim + 2] = acc[14]; }
 }
 
 // Backward, stage 2: one thread per primitive sums the slices (fixed order: deterministic) and
@@ -253,14 +357,26 @@ __global__ void pose_bwd_final_kernel(const float* __restrict__ q, const float* 
 #pragma unroll
     for (int i = 0; i < 15; ++i) acc[i] += p[i];
   }
-  if (gq) {
-    Pose pose; make_pose(q + 4 * (size_t)prim, pose);
-    float g4[4]; pose_backward(q + 4 * (size_t)prim, pose, acc, g4);
+  pose_bwd_chain(q, acc, prim, gv, gq, gt);
+}
+
+// Mixed assembly: primitive prim's slots start at slot prim * stride; it sums the slices_for(N of its kind) slots its
+// partial CTAs wrote, in the order pose_bwd_final_kernel sums them.
+__global__ void pose_mixed_bwd_final_kernel(const float* __restrict__ q, const float* __restrict__ partial,
+                                            float* __restrict__ gv, float* __restrict__ gq, float* __restrict__ gt,
+                                            int nprim, int K, int Kc, int ns_c, int ns_s, int stride) {
+  int prim = blockIdx.x * blockDim.x + threadIdx.x;
+  if (prim >= nprim) return;
+  const int nslices = (prim % K) < Kc ? ns_c : ns_s;
+  float acc[15];
 #pragma unroll
-    for (int i = 0; i < 4; ++i) gq[4 * (size_t)prim + i] = g4[i];
+  for (int i = 0; i < 15; ++i) acc[i] = 0.f;
+  for (int s = 0; s < nslices; ++s) {
+    const float* p = partial + ((size_t)prim * stride + s) * 16;
+#pragma unroll
+    for (int i = 0; i < 15; ++i) acc[i] += p[i];
   }
-  if (gt) { gt[3 * (size_t)prim] = acc[9]; gt[3 * (size_t)prim + 1] = acc[10]; gt[3 * (size_t)prim + 2] = acc[11]; }
-  if (gv) { gv[3 * (size_t)prim] = acc[12]; gv[3 * (size_t)prim + 1] = acc[13]; gv[3 * (size_t)prim + 2] = acc[14]; }
+  pose_bwd_chain(q, acc, prim, gv, gq, gt);
 }
 
 __global__ void cuboid_counts_kernel(const float* __restrict__ v, int* __restrict__ counts, int nprim, int N) {
@@ -348,6 +464,73 @@ extern "C" int vpn_pose_points_bwd(int kind, const float* v, const float* q, con
   pose_bwd_final_kernel<<<(nprim + 127) / 128, 128, 0, s>>>(q, workspace, kind == KIND_POINTS ? nullptr : grad_v,
                                                               grad_q, grad_t, nprim, ns);
   return vpn_check_launch("pose_bwd_final_kernel");
+}
+
+// Mixed cuboid + sphere assemblies: primitive b*K + k is a cuboid when k < Kc, else a sphere.
+// mode 0 = sampled: src_c = cuboid uniforms (B,Kc,N,3), src_s = sphere uniforms (B,K-Kc,N,2), Nc = Ns = N;
+// mode 1 = template: src_c = cuboid template (Nc,3), src_s = sphere template (Ns,3).
+// out (B, Kc*Nc + (K-Kc)*Ns, 3).  A kind without primitives may pass a NULL source.
+static int mixed_args(const char* what, int mode, int B, int K, int Kc, int Nc, int Ns, const float* src_c,
+                      const float* src_s) {
+  if (mode != 0 && mode != 1) { vpn_set_error("%s: mode must be 0 (sampled) or 1 (template)", what); return VPN_ERR_ARG; }
+  if (B <= 0 || K <= 0 || Nc <= 0 || Ns <= 0 || Kc < 0 || Kc > K || (mode == 0 && Nc != Ns)) {
+    vpn_set_error("%s: bad shape B=%d K=%d Kc=%d Nc=%d Ns=%d", what, B, K, Kc, Nc, Ns);
+    return VPN_ERR_SHAPE;
+  }
+  if ((Kc > 0 && !src_c) || (Kc < K && !src_s)) { vpn_set_error("%s: null source for a kind that is present", what); return VPN_ERR_ARG; }
+  return VPN_OK;
+}
+
+static int mixed_slices(int K, int Kc, int Nc, int Ns) {
+  return max(Kc > 0 ? slices_for(Nc) : 0, Kc < K ? slices_for(Ns) : 0);
+}
+
+// 16-byte accesses when every primitive's rows start on a 16-byte boundary: point counts of the present kinds divisible
+// by 4 (row offsets are then multiples of 4 points) and aligned base pointers.
+static int mixed_vec_ok(int K, int Kc, int Nc, int Ns, const float* src_c, const float* src_s, const float* rows) {
+  auto al = [](const float* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
+  return (Kc == 0 || (Nc % 4 == 0 && al(src_c))) && (Kc == K || (Ns % 4 == 0 && al(src_s))) && al(rows);
+}
+
+extern "C" int vpn_pose_mixed_fwd(int mode, const float* v, const float* q, const float* t, const float* src_c,
+                                  const float* src_s, float* out, int B, int K, int Kc, int Nc, int Ns, void* stream) {
+  int rc = mixed_args("pose mixed fwd", mode, B, K, Kc, Nc, Ns, src_c, src_s);
+  if (rc) return rc;
+  if (!v || !q || !out) { vpn_set_error("pose mixed fwd: null pointer"); return VPN_ERR_ARG; }
+  dim3 grid(B * K, mixed_slices(K, Kc, Nc, Ns)), block(kPoseThreads);
+  cudaStream_t s = (cudaStream_t)stream;
+  int vec_ok = mixed_vec_ok(K, Kc, Nc, Ns, src_c, src_s, out);
+  if (mode == 1) launch_pdl(pose_mixed_fwd_kernel<true>, grid, block, 0, s, v, q, t, src_c, src_s, out, K, Kc, Nc, Ns, vec_ok);
+  else           launch_pdl(pose_mixed_fwd_kernel<false>, grid, block, 0, s, v, q, t, src_c, src_s, out, K, Kc, Nc, Ns, vec_ok);
+  return vpn_check_launch("pose_mixed_fwd_kernel");
+}
+
+extern "C" int vpn_pose_mixed_bwd_workspace_floats(int B, int K, int Kc, int Nc, int Ns, size_t* floats) {
+  if (B <= 0 || K <= 0 || Nc <= 0 || Ns <= 0 || Kc < 0 || Kc > K) { vpn_set_error("pose mixed workspace: bad shape"); return VPN_ERR_SHAPE; }
+  if (!floats) { vpn_set_error("pose mixed workspace: null pointer"); return VPN_ERR_ARG; }
+  *floats = (size_t)B * K * mixed_slices(K, Kc, Nc, Ns) * 16;
+  return VPN_OK;
+}
+
+// grad_out (B, Kc*Nc + (K-Kc)*Ns, 3) -> grad_v (B*K,3), grad_q (B*K,4), grad_t (B*K,3); any may be NULL.
+extern "C" int vpn_pose_mixed_bwd(int mode, const float* v, const float* q, const float* src_c, const float* src_s,
+                                  const float* grad_out, float* grad_v, float* grad_q, float* grad_t, float* workspace,
+                                  size_t workspace_floats, int B, int K, int Kc, int Nc, int Ns, void* stream) {
+  int rc = mixed_args("pose mixed bwd", mode, B, K, Kc, Nc, Ns, src_c, src_s);
+  if (rc) return rc;
+  if (!v || !q || !grad_out || !workspace) { vpn_set_error("pose mixed bwd: null pointer"); return VPN_ERR_ARG; }
+  const int ns = mixed_slices(K, Kc, Nc, Ns), nprim = B * K;
+  if (workspace_floats < (size_t)nprim * ns * 16) { vpn_set_error("pose mixed bwd: workspace too small"); return VPN_ERR_WORKSPACE; }
+  dim3 grid(nprim, ns), block(kPoseThreads);
+  cudaStream_t s = (cudaStream_t)stream;
+  int vec_ok = mixed_vec_ok(K, Kc, Nc, Ns, src_c, src_s, grad_out);
+  if (mode == 1) pose_mixed_bwd_partial_kernel<true><<<grid, block, 0, s>>>(v, q, src_c, src_s, grad_out, workspace, K, Kc, Nc, Ns, vec_ok);
+  else           pose_mixed_bwd_partial_kernel<false><<<grid, block, 0, s>>>(v, q, src_c, src_s, grad_out, workspace, K, Kc, Nc, Ns, vec_ok);
+  rc = vpn_check_launch("pose_mixed_bwd_partial_kernel");
+  if (rc) return rc;
+  pose_mixed_bwd_final_kernel<<<(nprim + 127) / 128, 128, 0, s>>>(q, workspace, grad_v, grad_q, grad_t, nprim, K, Kc,
+                                                                    slices_for(Nc), slices_for(Ns), ns);
+  return vpn_check_launch("pose_mixed_bwd_final_kernel");
 }
 
 extern "C" int vpn_cuboid_face_counts(const float* v, int* counts, int nprim, int N, void* stream) {

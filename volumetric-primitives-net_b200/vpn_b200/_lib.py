@@ -27,6 +27,9 @@ _SIGNATURES = {
                                           c_int, POINTER(c_float), c_void_p]),
     "vpn_pose_bwd_workspace_floats": (c_int, [c_int, c_int, POINTER(c_size_t)]),
     "vpn_pose_points_bwd": (c_int, [c_int] + [c_void_p] * 9 + [c_size_t, c_int, c_int, c_void_p]),
+    "vpn_pose_mixed_fwd": (c_int, [c_int] + [c_void_p] * 6 + [c_int] * 5 + [c_void_p]),
+    "vpn_pose_mixed_bwd_workspace_floats": (c_int, [c_int] * 5 + [POINTER(c_size_t)]),
+    "vpn_pose_mixed_bwd": (c_int, [c_int] + [c_void_p] * 9 + [c_size_t] + [c_int] * 5 + [c_void_p]),
     "vpn_cuboid_face_counts": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "vpn_view_workspace_bytes": (c_int, [c_int, POINTER(c_size_t)]),
     "vpn_view_points": (c_int, [c_int, c_int] + [c_void_p] * 7 + [c_size_t, c_int, c_int, c_void_p]),

@@ -105,6 +105,79 @@ def mesh_vertices(template: torch.Tensor, v: torch.Tensor, q: torch.Tensor, t: t
     return out.view(b, k * nv, 3)
 
 
+MIXED_SAMPLED, MIXED_TEMPLATE = 0, 1
+
+
+class _PoseMixed(torch.autograd.Function):
+    """A mixed assembly of K primitives per sample, primitive k a cuboid when k < kc, else a sphere: out (B, kc*nc +
+    (K-kc)*ns, 3), each primitive's rows posed from src_c (cuboids) or src_s (spheres) as _PosePoints does for its kind."""
+
+    @staticmethod
+    def forward(ctx, mode, b, k, kc, nc, ns, v, q, t, src_c, src_s):
+        lib = _lib.load()
+        v, q, t = require(v, f32, "v"), require(q, f32, "q"), require(t, f32, "t")
+        src_c, src_s = require(src_c, f32, "cuboid source"), require(src_s, f32, "sphere source")
+        dev = q.device
+        out = torch.empty((b, kc * nc + (k - kc) * ns, 3), dtype=f32, device=dev)
+        check(lib.vpn_pose_mixed_fwd(mode, ptr(v), ptr(q), ptr(t), ptr(src_c), ptr(src_s), ptr(out), b, k, kc, nc, ns,
+                                     stream_ptr(dev)), "vpn_pose_mixed_fwd")
+        ctx.dims = (mode, b, k, kc, nc, ns)
+        ctx.save_for_backward(v, q, src_c, src_s)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        lib = _lib.load()
+        v, q, src_c, src_s = ctx.saved_tensors
+        mode, b, k, kc, nc, ns = ctx.dims
+        dev = q.device
+        grad_out = grad_out.contiguous()
+        need_v, need_q, need_t = ctx.needs_input_grad[6:9]
+        gv = torch.empty((b * k, 3), dtype=f32, device=dev) if need_v else None
+        gq = torch.empty((b * k, 4), dtype=f32, device=dev) if need_q else None
+        gt = torch.empty((b * k, 3), dtype=f32, device=dev) if need_t else None
+        nfl = ctypes.c_size_t(0)
+        check(lib.vpn_pose_mixed_bwd_workspace_floats(b, k, kc, nc, ns, ctypes.byref(nfl)), "vpn_pose_mixed_bwd_workspace_floats")
+        ws = torch.empty(max(nfl.value, 16), dtype=f32, device=dev)
+        check(lib.vpn_pose_mixed_bwd(mode, ptr(v), ptr(q), ptr(src_c), ptr(src_s), ptr(grad_out), ptr(gv), ptr(gq), ptr(gt),
+                                     ptr(ws), nfl.value, b, k, kc, nc, ns, stream_ptr(dev)), "vpn_pose_mixed_bwd")
+        return (None,) * 6 + (gv, gq, gt, None, None)
+
+
+def sample_mixed_primitives(n_cuboids: int, v: torch.Tensor, q: torch.Tensor, t: torch.Tensor, u_cuboid: torch.Tensor,
+                            u_sphere: torch.Tensor) -> torch.Tensor:
+    """Fused sampling + pose of a mixed assembly, train.py:105-120 with CUBOID_NUM = n_cuboids and SPHERE_NUM = K -
+    n_cuboids, in one launch: primitive k is a cuboid when k < n_cuboids, else a sphere.
+
+    v (B,K,3), q (B,K,4), t (B,K,3); u_cuboid (B,n_cuboids,N,3), u_sphere (B,K-n_cuboids,N,2), uniforms of sample_primitives.
+    Returns (B, K*N, 3), primitive-major: the cuboids' points, then the spheres', each primitive's the bits
+    sample_primitives gives for its kind."""
+    b, k, vf, qf, tf = _flat_prims(v, q, t)
+    kc = int(n_cuboids)
+    assert 0 <= kc <= k, f"n_cuboids must be in [0, K = {k}], got {kc}"
+    assert u_cuboid.dim() == 4 and tuple(u_cuboid.shape[:2]) == (b, kc) and u_cuboid.size(-1) == 3, (
+        f"cuboid uniforms must be (B, n_cuboids, N, 3) = ({b}, {kc}, N, 3), got {tuple(u_cuboid.shape)}")
+    assert u_sphere.dim() == 4 and tuple(u_sphere.shape[:2]) == (b, k - kc) and u_sphere.size(-1) == 2, (
+        f"sphere uniforms must be (B, K - n_cuboids, N, 2) = ({b}, {k - kc}, N, 2), got {tuple(u_sphere.shape)}")
+    n = u_cuboid.size(2)
+    assert u_sphere.size(2) == n and n > 0, "cuboid and sphere uniforms must have the same N > 0"
+    return _PoseMixed.apply(MIXED_SAMPLED, b, k, kc, n, n, vf, qf, tf, u_cuboid.contiguous(), u_sphere.contiguous())
+
+
+def mesh_vertices_mixed(n_cuboids: int, cuboid_template: torch.Tensor, sphere_template: torch.Tensor, v: torch.Tensor,
+                        q: torch.Tensor, t: torch.Tensor) -> torch.Tensor:
+    """Vertices of a mixed assembly's meshes in one launch: primitive k posed from the cuboid template (Vc,3) when
+    k < n_cuboids, else from the sphere template (Vs,3).  Returns (B, n_cuboids*Vc + (K-n_cuboids)*Vs, 3) in compose
+    order (meshing.py:28-46), each primitive's the bits mesh_vertices gives for its template."""
+    b, k, vf, qf, tf = _flat_prims(v, q, t)
+    kc = int(n_cuboids)
+    assert 0 <= kc <= k, f"n_cuboids must be in [0, K = {k}], got {kc}"
+    for tpl in (cuboid_template, sphere_template):
+        assert tpl.dim() == 2 and tpl.size(1) == 3 and tpl.size(0) > 0, "templates must be (V, 3)"
+    return _PoseMixed.apply(MIXED_TEMPLATE, b, k, kc, cuboid_template.size(0), sphere_template.size(0), vf, qf, tf,
+                            cuboid_template.contiguous(), sphere_template.contiguous())
+
+
 def transform_points(points: torch.Tensor, q: torch.Tensor, t: Optional[torch.Tensor]) -> torch.Tensor:
     """translate(rotate(points, q), t)  (transform/transform.py:6-9); t=None -> rotate only."""
     assert points.dim() == 3 and points.size(-1) == 3

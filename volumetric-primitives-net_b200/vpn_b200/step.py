@@ -21,7 +21,7 @@ from . import ops, templates
 
 @dataclass
 class PrimitiveLossConfig:
-    kind: str = "sphere"              # 'sphere' | 'cuboid'   (config.py:32-35 SPHERE_NUM / CUBOID_NUM)
+    kind: str = "sphere"              # 'sphere' | 'cuboid' | 'mixed'   (config.py:32-35 SPHERE_NUM / CUBOID_NUM)
     l_view_cd: float = 1.0            # config.py:14-17
     l_can_cd: float = 0.0
     l_sil: float = 0.0
@@ -40,6 +40,14 @@ class PrimitiveLossConfig:
     l_emd: float = 0.0
     emd_eps: float = 0.005            # train.py:188-195
     emd_iters: int = 50
+    # kind = 'mixed': primitive k of every sample is a cuboid when k < n_cuboids, else a sphere (train.py with
+    # CUBOID_NUM = n_cuboids, SPHERE_NUM = K - n_cuboids).  Uniforms are then the pair (u_cuboid, u_sphere).
+    n_cuboids: int = 0
+
+    def __post_init__(self):
+        assert self.kind in ("sphere", "cuboid", "mixed"), f"kind must be 'sphere', 'cuboid' or 'mixed', got {self.kind!r}"
+        assert self.n_cuboids >= 0, "n_cuboids must be >= 0"
+        assert self.kind == "mixed" or self.n_cuboids == 0, "n_cuboids is for kind='mixed' only"
 
 
 class _LossStep:
@@ -136,17 +144,45 @@ def _capture(run, device, warmup: int):
 class PrimitiveLoss(_LossStep):
     def __init__(self, config: Optional[PrimitiveLossConfig] = None):
         self.cfg = config or PrimitiveLossConfig()
-        assert self.cfg.kind in ("sphere", "cuboid")
+        assert self.cfg.kind in ("sphere", "cuboid", "mixed")
+
+    def _kinds(self, k: int):
+        """Template name of each of the K primitives of a sample."""
+        cfg = self.cfg
+        if cfg.kind != "mixed":
+            return [cfg.kind] * k
+        assert cfg.n_cuboids <= k, f"n_cuboids = {cfg.n_cuboids} exceeds the K = {k} primitives"
+        return ["cuboid"] * cfg.n_cuboids + ["sphere"] * (k - cfg.n_cuboids)
 
     def composed_faces(self, k: int, device) -> torch.Tensor:
-        """Faces of K composed template meshes (meshing.py:28-46 running vertex offset), int32 (K*F,3)."""
+        """Faces of K composed template meshes (meshing.py:28-46 running vertex offset), int32 (sum of F,3); under 'mixed'
+        the n_cuboids cuboids' faces come first, then the spheres'."""
         key = (k, str(device))
         cache = self.__dict__.setdefault("_faces", {})
         if key not in cache:
-            tv, tf = templates.template(self.cfg.kind, device)
-            nv = tv.shape[0]
-            cache[key] = torch.cat([tf + i * nv for i in range(k)], dim=0).contiguous()
+            faces, off = [], 0
+            for name in self._kinds(k):
+                tv, tf = templates.template(name, device)
+                faces.append(tf + off)
+                off += tv.shape[0]
+            cache[key] = torch.cat(faces, dim=0).contiguous()
         return cache[key]
+
+    def _vertices(self, v, q, t):
+        """Composed template vertices of every primitive, (B, sum of V, 3)."""
+        cfg = self.cfg
+        if cfg.kind == "mixed":
+            return ops.mesh_vertices_mixed(cfg.n_cuboids, templates.template("cuboid", v.device)[0],
+                                           templates.template("sphere", v.device)[0], v, q, t)
+        return ops.mesh_vertices(templates.template(cfg.kind, v.device)[0], v, q, t)
+
+    def _points_per_sample(self, k: int, uniforms) -> int:
+        """Points per sample the Chamfer / EMD terms see, from the shapes alone."""
+        if self.cfg.vertex_chamfer:
+            return sum(templates.template(name, "cpu")[0].shape[0] for name in self._kinds(k))
+        if self.cfg.kind == "mixed":
+            return k * uniforms[0].shape[2]
+        return k * uniforms.shape[2]
 
     def __call__(self, v: torch.Tensor, q: torch.Tensor, t: torch.Tensor, uniforms: torch.Tensor,
                  view_center_points: torch.Tensor, silhouettes: Optional[torch.Tensor] = None,
@@ -159,15 +195,20 @@ class PrimitiveLoss(_LossStep):
         cfg = self.cfg
         out: Dict[str, torch.Tensor] = {}
         b, k = q.shape[:2]
+        if cfg.kind == "mixed":
+            self._kinds(k)
+            assert cfg.vertex_chamfer or (isinstance(uniforms, (tuple, list)) and len(uniforms) == 2), (
+                "kind='mixed' takes uniforms = (u_cuboid, u_sphere)")
         if cfg.l_emd:
             # the auction pairs every point with one target (emd_module.py:37-38): checked from the shapes before any launch
-            per_prim = templates.template(cfg.kind, v.device)[0].shape[0] if cfg.vertex_chamfer else uniforms.shape[2]
-            assert view_center_points.dim() == 3 and tuple(view_center_points.shape) == (b, k * per_prim, 3), (
-                f"l_emd needs as many points as targets: {k} x {per_prim} points, targets {tuple(view_center_points.shape)}")
+            n_points = self._points_per_sample(k, uniforms)
+            assert view_center_points.dim() == 3 and tuple(view_center_points.shape) == (b, n_points, 3), (
+                f"l_emd needs as many points as targets: {n_points} points, targets {tuple(view_center_points.shape)}")
         verts = None
         if cfg.vertex_chamfer:
-            tv, _ = templates.template(cfg.kind, v.device)
-            points = verts = ops.mesh_vertices(tv, v, q, t)
+            points = verts = self._vertices(v, q, t)
+        elif cfg.kind == "mixed":
+            points = ops.sample_mixed_primitives(cfg.n_cuboids, v, q, t, uniforms[0], uniforms[1])
         else:
             points = ops.sample_primitives(cfg.kind, v, q, t, uniforms)
         out["points"] = points
@@ -225,8 +266,7 @@ class PrimitiveLoss(_LossStep):
         cfg = self.cfg
         b, k = q.shape[:2]
         if verts is None:
-            tv, _ = templates.template(cfg.kind, v.device)
-            verts = ops.mesh_vertices(tv, v, q, t)
+            verts = self._vertices(v, q, t)
         faces = self.composed_faces(k, v.device)
         h, w = silhouettes.shape[-2:]
         if sil_cameras is None:
@@ -268,11 +308,25 @@ class GraphedPrimitiveLoss:
         self.canonical = None if canonical_points is None else canonical_points.detach().clone()
         self.cameras = None if cameras is None else tuple(c.detach().clone() for c in cameras)
         b, k = q.shape[:2]
-        self.ushape = None if config.vertex_chamfer else (b, k, n_samples, 2 if config.kind == "sphere" else 3)
+        if config.vertex_chamfer:
+            self.ushape = None
+        elif config.kind == "mixed":
+            kc = config.n_cuboids
+            assert kc <= k, f"n_cuboids = {kc} exceeds the K = {k} primitives"
+            self.ushape = ((b, kc, n_samples, 3), (b, k - kc, n_samples, 2))      # u_cuboid, then u_sphere
+        else:
+            self.ushape = (b, k, n_samples, 2 if config.kind == "sphere" else 3)
         assert config.vertex_chamfer or n_samples > 0, "n_samples (points per primitive) is required unless vertex_chamfer"
 
+        def draw():
+            if self.ushape is None:
+                return None
+            if config.kind == "mixed":
+                return tuple(torch.rand(shape, device=dev) for shape in self.ushape)
+            return torch.rand(self.ushape, device=dev)
+
         def run():
-            u = None if self.ushape is None else torch.rand(self.ushape, device=dev)      # drawn on the device, as the reference does
+            u = draw()      # drawn on the device, as the reference does
             cams = self.cameras or (None, None, None, None)
             out = self.step(self.v, self.q, self.t, u, self.targets, silhouettes=self.sil, canonical_points=self.canonical,
                             dists=cams[0], elevs=cams[1], azims=cams[2], angles=cams[3])
