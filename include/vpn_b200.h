@@ -132,6 +132,14 @@ int vpn_chamfer_loss_fwd(const float* min1, const float* min2, float w1, float w
 int vpn_chamfer_loss_bwd(const float* p1, const float* p2, const float* min1, const int* idx1,
                          const float* min2, const int* idx2, const float* grad_loss, float w1, float w2,
                          float* grad_p1, float* grad_p2, int B, int P, int M, void* stream);
+/* The same head with the batch mean inside: loss (1 float) = weight * mean_b(w1*mean(min1[b]) + w2*mean(min2[b])), the
+ * per-sample values summed in a fixed order.  The backward reads the scalar upstream gradient grad_loss (1 float) on the
+ * device and scales it as autograd does through torch's `loss.mean() * weight`.  B >= 1. */
+int vpn_chamfer_loss_mean_fwd(const float* min1, const float* min2, float w1, float w2, float weight, float* loss,
+                              float* scratch /* >= 64*B floats */, int B, int P, int M, void* stream);
+int vpn_chamfer_loss_mean_bwd(const float* p1, const float* p2, const float* min1, const int* idx1,
+                              const float* min2, const int* idx2, const float* grad_loss, float w1, float w2, float weight,
+                              float* grad_p1, float* grad_p2, int B, int P, int M, void* stream);
 
 /* ---- soft silhouette (modules/loss/silhouette.py:13-23 -> render/vertex_renderer.py:15-26 -> kaolin DIB-R)
  * verts (B,V,3), faces (F,3) int32 shared topology, cam_rot (B,3,3), cam_pos (B,3), proj = (px,py,pz).

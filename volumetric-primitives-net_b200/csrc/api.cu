@@ -27,7 +27,7 @@ int vpn_check_launch(const char* what) {
 namespace vpn {
 int chamfer_simple_direction(const float* A, const float* Bp, float* mn, int* idx, u64* key,
                              int B, int nA, int nB, int sm_count, cudaStream_t s);
-int chamfer_smallp(const float* p1, const float* p2, float* min1, int* idx1, float* min2, int* idx2, u64* key1,
+int chamfer_smallp(const float* p1, const float* p2, float* min1, int* idx1, float* min2, int* idx2,
                    int B, int P, int M, cudaStream_t s);
 int chamfer_smallp_limit();
 int chamfer_tiled_supported(int B, int P, int M, int mode);
@@ -112,7 +112,7 @@ static int chamfer_fwd_impl(const float* p1, const float* p2, float* min1, int* 
   if (workspace_bytes < need) { vpn_set_error("chamfer fwd: workspace too small (%zu < %zu)", workspace_bytes, need); return VPN_ERR_WORKSPACE; }
   vpn::u64* key1 = reinterpret_cast<vpn::u64*>(workspace);
   vpn::u64* key2 = reinterpret_cast<vpn::u64*>(reinterpret_cast<char*>(workspace) + align256((size_t)B * P * 8));
-  if (impl == 0 && P <= vpn::chamfer_smallp_limit() && !ev) return vpn::chamfer_smallp(p1, p2, min1, idx1, min2, idx2, key1, B, P, M, s);
+  if (impl == 0 && P <= vpn::chamfer_smallp_limit() && !ev) return vpn::chamfer_smallp(p1, p2, min1, idx1, min2, idx2, B, P, M, s);
   if (ev) { cudaEventRecord(ev[0], s); }
   int rc = vpn::chamfer_simple_direction(p1, p2, min1, idx1, key1, B, P, M, sm_count(), s);
   if (rc) return rc;
@@ -151,7 +151,7 @@ extern "C" const char* vpn_chamfer_main_kernel(int B, int P, int M, int impl) {
   if (impl < 0 || impl > 5 || B <= 0 || P <= 0 || M <= 0) return "invalid";
   if (impl != 1 && vpn::chamfer_tiled_supported(B, P, M, impl_mode(impl)))
     return vpn::chamfer_tiled_uses_tc(B, P, M, impl_mode(impl)) ? "chamfer_tc_kernel" : "chamfer_tiled_kernel";
-  if (impl == 0 && P <= vpn::chamfer_smallp_limit()) return "chamfer_smallp_kernel";
+  if (impl == 0 && P <= vpn::chamfer_smallp_limit()) return "chamfer_smallp_fwd_kernel";
   return "chamfer_simple_kernel";
 }
 

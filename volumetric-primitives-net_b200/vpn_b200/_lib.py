@@ -45,6 +45,10 @@ _SIGNATURES = {
     "vpn_chamfer_loss_fwd": (c_int, [c_void_p, c_void_p, c_float, c_float, c_void_p, c_void_p, c_int, c_int, c_int,
                                      c_void_p]),
     "vpn_chamfer_loss_bwd": (c_int, [c_void_p] * 7 + [c_float, c_float, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
+    "vpn_chamfer_loss_mean_fwd": (c_int, [c_void_p, c_void_p, c_float, c_float, c_float, c_void_p, c_void_p, c_int, c_int,
+                                          c_int, c_void_p]),
+    "vpn_chamfer_loss_mean_bwd": (c_int, [c_void_p] * 7 + [c_float, c_float, c_float, c_void_p, c_void_p, c_int, c_int, c_int,
+                                                           c_void_p]),
     "vpn_silhouette_workspace_bytes": (c_int, [c_int, c_int, c_int, POINTER(c_size_t)]),
     "vpn_silhouette_fwd": (c_int, [c_void_p] * 4 + [c_float] * 4 + [c_int, c_float, c_float, c_int] + [c_void_p] * 4
                            + [c_size_t] + [c_int] * 5 + [c_void_p]),

@@ -325,10 +325,11 @@ def chamfer_nn_stage_ms(points1: torch.Tensor, points2: torch.Tensor, impl: int 
 
 class _ChamferLoss(torch.autograd.Function):
     """Per-sample loss w1*mean(min1) + w2*mean(min2) with the nearest-neighbour search, the two means and the
-    whole backward as vpn_b200 kernels (no (B,P)/(B,M) gradient tensors, no elementwise torch launches)."""
+    whole backward as vpn_b200 kernels (no (B,P)/(B,M) gradient tensors, no elementwise torch launches).
+    mean=True: the scalar weight * mean over the batch instead, also in the loss head's kernels."""
 
     @staticmethod
-    def forward(ctx, p1, p2, w1, w2, impl):
+    def forward(ctx, p1, p2, w1, w2, impl, mean, weight):
         lib = _lib.load()
         p1 = require(p1.contiguous(), f32, "points1")
         p2 = require(p2.contiguous(), f32, "points2")
@@ -343,12 +344,18 @@ class _ChamferLoss(torch.autograd.Function):
         st = stream_ptr(dev)
         check(lib.vpn_chamfer_fwd(ptr(p1), ptr(p2), ptr(min1), ptr(idx1), ptr(min2), ptr(idx2), b, p, m,
                                   ptr(ws), nb.value, impl, st), "vpn_chamfer_fwd")
-        loss = torch.empty((b,), dtype=f32, device=dev)
         part = torch.empty((b * 64,), dtype=f32, device=dev)
-        check(lib.vpn_chamfer_loss_fwd(ptr(min1), ptr(min2), float(w1), float(w2), ptr(loss), ptr(part), b, p, m, st),
-              "vpn_chamfer_loss_fwd")
+        if mean:
+            loss = torch.empty((), dtype=f32, device=dev)
+            check(lib.vpn_chamfer_loss_mean_fwd(ptr(min1), ptr(min2), float(w1), float(w2), float(weight), ptr(loss),
+                                                ptr(part), b, p, m, st), "vpn_chamfer_loss_mean_fwd")
+        else:
+            loss = torch.empty((b,), dtype=f32, device=dev)
+            check(lib.vpn_chamfer_loss_fwd(ptr(min1), ptr(min2), float(w1), float(w2), ptr(loss), ptr(part), b, p, m, st),
+                  "vpn_chamfer_loss_fwd")
         ctx.save_for_backward(p1, p2, min1, idx1, min2, idx2)
         ctx.w = (float(w1), float(w2))
+        ctx.mean_weight = float(weight) if mean else None
         return loss
 
     @staticmethod
@@ -361,19 +368,28 @@ class _ChamferLoss(torch.autograd.Function):
         gloss = gloss.contiguous()
         gp1 = torch.empty_like(p1)
         gp2 = torch.empty_like(p2) if ctx.needs_input_grad[1] else None
-        check(lib.vpn_chamfer_loss_bwd(ptr(p1), ptr(p2), ptr(min1), ptr(idx1), ptr(min2), ptr(idx2), ptr(gloss),
-                                       ctx.w[0], ctx.w[1], ptr(gp1), ptr(gp2), b, p, m, stream_ptr(dev)),
-              "vpn_chamfer_loss_bwd")
-        return (gp1 if ctx.needs_input_grad[0] else None), gp2, None, None, None
+        if ctx.mean_weight is None:
+            check(lib.vpn_chamfer_loss_bwd(ptr(p1), ptr(p2), ptr(min1), ptr(idx1), ptr(min2), ptr(idx2), ptr(gloss),
+                                           ctx.w[0], ctx.w[1], ptr(gp1), ptr(gp2), b, p, m, stream_ptr(dev)),
+                  "vpn_chamfer_loss_bwd")
+        else:
+            check(lib.vpn_chamfer_loss_mean_bwd(ptr(p1), ptr(p2), ptr(min1), ptr(idx1), ptr(min2), ptr(idx2), ptr(gloss),
+                                                ctx.w[0], ctx.w[1], ctx.mean_weight, ptr(gp1), ptr(gp2), b, p, m,
+                                                stream_ptr(dev)), "vpn_chamfer_loss_mean_bwd")
+        return (gp1 if ctx.needs_input_grad[0] else None), gp2, None, None, None, None, None
 
 
-def chamfer_distance(points1, points2, each_batch=False, w1=1.0, w2=1.0, impl: int = CHAMFER_AUTO):
-    """ChamferDistanceLoss.forward (chamfer_distance.py:10-30)."""
+def chamfer_distance(points1, points2, each_batch=False, w1=1.0, w2=1.0, impl: int = CHAMFER_AUTO, weight: float = 1.0):
+    """ChamferDistanceLoss.forward (chamfer_distance.py:10-30) times `weight`.  The default (each_batch=False) returns
+    weight * the batch mean, computed in the loss head's kernels with a fixed summation order; its gradients are the bits
+    of `chamfer_distance(..., each_batch=True).mean() * weight`.  each_batch=True returns the per-sample (B,) values."""
     assert points1.dim() == 3 and points1.size(-1) == 3          # chamfer_distance.py:33-35
     assert points2.dim() == 3 and points2.size(-1) == 3
     assert points1.size(0) == points2.size(0)
-    loss = _ChamferLoss.apply(points1, points2, w1, w2, impl)
-    return loss if each_batch else loss.mean()
+    if each_batch:
+        loss = _ChamferLoss.apply(points1, points2, w1, w2, impl, False, 1.0)
+        return loss if weight == 1.0 else loss * weight
+    return _ChamferLoss.apply(points1, points2, w1, w2, impl, True, weight)
 
 
 # --------------------------------------------------------------------------------------

@@ -240,14 +240,14 @@ class PrimitiveLoss(_LossStep):
             emd_term, emd_side = self._emd_branch(points, view_center_points)
         if cfg.l_view_cd:
             add("view_cd", ops.chamfer_distance(points, view_center_points, w1=cfg.cd_w1, w2=cfg.cd_w2,
-                                                impl=cfg.chamfer_impl) * cfg.l_view_cd)
+                                                impl=cfg.chamfer_impl, weight=cfg.l_view_cd))
         if cfg.l_can_cd:
             can = ops.view_to_obj_points(points, dists, elevs, azims, angles)
             add("obj_cd", ops.chamfer_distance(can, canonical_points, w1=cfg.cd_w1, w2=cfg.cd_w2,
-                                               impl=cfg.chamfer_impl) * cfg.l_can_cd)
+                                               impl=cfg.chamfer_impl, weight=cfg.l_can_cd))
         if cfg.l_vp_div:
             add("vp_div", ops.chamfer_distance(t.contiguous(), view_center_points, w1=0.5, w2=1.0,
-                                               impl=cfg.chamfer_impl) * cfg.l_vp_div)
+                                               impl=cfg.chamfer_impl, weight=cfg.l_vp_div))
         if emd_term is not None:
             self._join(v.device, emd_side)
             add("emd", emd_term)
@@ -325,12 +325,16 @@ class GraphedPrimitiveLoss:
                 return tuple(torch.rand(shape, device=dev) for shape in self.ushape)
             return torch.rand(self.ushape, device=dev)
 
+        # seeds autograd.grad of the total: made once, outside the capture, so a replay has no fill kernel for it.  The
+        # graph reads it at every replay, so the object keeps it alive.
+        self._one = torch.ones((), device=dev)
+
         def run():
             u = draw()      # drawn on the device, as the reference does
             cams = self.cameras or (None, None, None, None)
             out = self.step(self.v, self.q, self.t, u, self.targets, silhouettes=self.sil, canonical_points=self.canonical,
                             dists=cams[0], elevs=cams[1], azims=cams[2], angles=cams[3])
-            gv, gq, gt = torch.autograd.grad(out["total"], (self.v, self.q, self.t))
+            gv, gq, gt = torch.autograd.grad(out["total"], (self.v, self.q, self.t), grad_outputs=self._one)
             if after_backward is not None:
                 after_backward()
             return out["total"], gv, gq, gt
@@ -438,7 +442,7 @@ class MeshLoss(_LossStep):
         if cfg.l_emd:
             emd_term, emd_side = self._emd_branch(points, targets)
         if cfg.l_cd:
-            add("cd", ops.chamfer_distance(points, targets, w1=cfg.cd_w1, w2=cfg.cd_w2, impl=cfg.chamfer_impl) * cfg.l_cd)
+            add("cd", ops.chamfer_distance(points, targets, w1=cfg.cd_w1, w2=cfg.cd_w2, impl=cfg.chamfer_impl, weight=cfg.l_cd))
         if emd_term is not None:
             self._join(verts.device, emd_side)
             add("emd", emd_term)
@@ -475,9 +479,11 @@ class GraphedMeshLoss:
         self.targets = targets.detach().clone()
         self.sil = None if silhouettes is None else silhouettes.detach().clone()
 
+        self._one = torch.ones((), device=dev)       # as in GraphedPrimitiveLoss
+
         def run():
             out = self.step(self.verts, self.faces, self.targets, silhouettes=self.sil)
-            (gv,) = torch.autograd.grad(out["total"], (self.verts,))
+            (gv,) = torch.autograd.grad(out["total"], (self.verts,), grad_outputs=self._one)
             return out["total"], gv
 
         # the sampler's backward reads the cached vertex CSR of these faces: build it before the capture and keep it
