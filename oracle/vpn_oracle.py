@@ -542,11 +542,120 @@ def project_vertices(verts: torch.Tensor, rot: torch.Tensor, pos: torch.Tensor):
     return cam, xyz[:, :, :2] / xyz[:, :, 2:3]
 
 
+def _sil_faces(verts, faces, rot, pos):
+    """Per-face screen data: s (B,F,3,2) scaled screen coordinates, front (B,F), live (B,F).
+    A face with a non-finite screen coordinate (a NaN vertex, or a vertex on the camera plane, cam.z = 0) is not live:
+    it takes part in neither pass, and its coordinates are replaced by 0 so that no NaN reaches the other faces'
+    gradients (only the offending vertex's own gradient is undefined)."""
+    cam, xy = project_vertices(verts, rot, pos)
+    p0c, p1c, p2c = cam[:, faces[:, 0]], cam[:, faces[:, 1]], cam[:, faces[:, 2]]       # (B,F,3)
+    normal_z = torch.cross(p1c - p0c, p2c - p0c, dim=2)[:, :, 2]                          # (B,F)
+    s = torch.stack([xy[:, faces[:, 0]], xy[:, faces[:, 1]], xy[:, faces[:, 2]]], dim=2) * DIBR_MULTIPLIER  # (B,F,3,2)
+    live = torch.isfinite(s).flatten(2).all(dim=2)
+    s = torch.where(live[:, :, None, None], s, torch.zeros_like(s))
+    return s, normal_z >= 0, live                          # direction < 0 -> skipped
+
+
+def _sil_pixel_centres(height: int, width: int, pixels=None):
+    """Scaled pixel centres X, Y (P,), flat index h*W+w; `pixels` selects a subset."""
+    mult = DIBR_MULTIPLIER
+    wi = torch.arange(width, dtype=torch.float32)
+    hi = torch.arange(height, dtype=torch.float32)
+    x0 = (mult / width) * (2 * wi + 1 - width)            # (W,)
+    y0 = (mult / height) * (height - 2 * hi - 1)          # (H,)
+    X = x0[None, :].expand(height, width).reshape(-1)     # (HW,)
+    Y = y0[:, None].expand(height, width).reshape(-1)
+    if pixels is not None:
+        X, Y = X[pixels], Y[pixels]
+    return X, Y
+
+
+@torch.no_grad()
+def _sil_select(sb, front, live, Xp, Yp, soft_cull_backfaces: bool, knum: int):
+    """Coverage and soft-candidate selection of one sample (no gradient).  sb (F,3,2); front, live (F,); Xp, Yp (P,1).
+    Returns covered (P,), in_soft (P,F) (expanded box holds the pixel) and use (P,F) (the first knum of those, in face
+    index order, on uncovered pixels)."""
+    ax, ay = sb[:, 0, 0][None], sb[:, 0, 1][None]          # (1,F)
+    bx, by = sb[:, 1, 0][None], sb[:, 1, 1][None]
+    cx, cy = sb[:, 2, 0][None], sb[:, 2, 1][None]
+    bmin = sb.min(dim=1)[0]
+    bmax = sb.max(dim=1)[0]
+    bmin2 = bmin - DIBR_EXPAND * DIBR_MULTIPLIER
+    bmax2 = bmax + DIBR_EXPAND * DIBR_MULTIPLIER
+    in_tight = (Xp >= bmin[:, 0][None]) & (Xp < bmax[:, 0][None]) & \
+               (Yp >= bmin[:, 1][None]) & (Yp < bmax[:, 1][None]) & live[None]
+    m_, p_, n_, q_ = bx - ax, by - ay, cx - ax, cy - ay
+    s_, t_ = Xp - ax, Yp - ay
+    k1 = s_ * q_ - n_ * t_
+    k2 = m_ * t_ - s_ * p_
+    k3 = m_ * q_ - n_ * p_
+    w1 = k1 / (k3 + DIBR_EPS)
+    w2 = k2 / (k3 + DIBR_EPS)
+    w0 = 1 - w1 - w2
+    inside = in_tight & front[None] & (w0 >= 0) & (w1 >= 0) & (w2 >= 0)
+    covered = inside.any(dim=1)                            # (P,)
+    in_soft = (Xp >= bmin2[:, 0][None]) & (Xp < bmax2[:, 0][None]) & \
+              (Yp >= bmin2[:, 1][None]) & (Yp < bmax2[:, 1][None]) & live[None]
+    if soft_cull_backfaces:
+        in_soft = in_soft & front[None]
+    rank = torch.cumsum(in_soft.to(torch.int32), dim=1)
+    use = in_soft & (rank <= knum) & (~covered)[:, None]
+    return covered, in_soft, use
+
+
+def _sil_dist2(sb, Xp, Yp):
+    """Squared distance pixel -> triangle, DIB-R's 6 cases: pd (P,F,6) (differentiable) and off (P,F,3), the edges whose
+    perpendicular foot falls off the segment (their case holds the constant 4 mult^2)."""
+    mult = DIBR_MULTIPLIER
+    vx = [sb[:, i, 0][None] for i in range(3)]              # (1,F)
+    vy = [sb[:, i, 1][None] for i in range(3)]
+    pd, off = [], []
+    for i in range(3):
+        x1, y1, x2, y2 = vx[i], vy[i], vx[(i + 1) % 3], vy[(i + 1) % 3]
+        A = y2 - y1
+        Bc = x1 - x2
+        C = x2 * y1 - x1 * y2
+        up = A * Xp + Bc * Yp + C
+        down = A * A + Bc * Bc
+        with torch.no_grad():
+            x3 = (Bc * Bc * Xp - A * Bc * Yp - A * C) / (down + DIBR_EPS)
+            y3 = (A * A * Yp - A * Bc * Xp - Bc * C) / (down + DIBR_EPS)
+            bad = ((x3 - x1) * (x3 - x2) + (y3 - y1) * (y3 - y2)) > 0
+        perp = up * up / (down + DIBR_EPS)
+        pd.append(torch.where(bad, torch.full_like(perp, 4 * mult * mult), perp))
+        off.append(bad)
+    for i in range(3):
+        pd.append((Xp - vx[i]) ** 2 + (Yp - vy[i]) ** 2)
+    return torch.stack(pd, dim=2), torch.stack(off, dim=2)
+
+
+@torch.no_grad()
+def soft_silhouette_selection(verts, faces, rot, pos, height: int, width: int, soft_cull_backfaces: bool = False,
+                              pixels=None, knum: int = DIBR_KNUM):
+    """The discrete choices soft_silhouette makes, for tests that need to know which faces a pixel used.  Per sample
+    (lists of length B): covered (P,), in_soft (P,F), use (P,F) as in _sil_select, case (P,F) the winning distance case
+    (0-2 edge i -> i+1, 3-5 vertex; first minimum) and const (P,F) True where that case is the foot-off constant."""
+    s, front, live = _sil_faces(verts, faces, rot, pos)
+    X, Y = _sil_pixel_centres(height, width, pixels)
+    Xp, Yp = X[:, None], Y[:, None]
+    out = {"covered": [], "in_soft": [], "use": [], "case": [], "const": []}
+    for bi in range(verts.shape[0]):
+        covered, in_soft, use = _sil_select(s[bi], front[bi], live[bi], Xp, Yp, soft_cull_backfaces, knum)
+        pd, off = _sil_dist2(s[bi], Xp, Yp)
+        case = torch.argmin(pd, dim=2)
+        const = (case < 3) & torch.gather(off, 2, case.clamp(max=2)[..., None]).squeeze(2)
+        for k, x in (("covered", covered), ("in_soft", in_soft), ("use", use), ("case", case), ("const", const)):
+            out[k].append(x)
+    return out
+
+
 def soft_silhouette(verts: torch.Tensor, faces: torch.Tensor, rot: torch.Tensor, pos: torch.Tensor,
-                    height: int, width: int, soft_cull_backfaces: bool = False, pixels=None) -> torch.Tensor:
+                    height: int, width: int, soft_cull_backfaces: bool = False, pixels=None,
+                    knum: int = DIBR_KNUM) -> torch.Tensor:
     """Soft alpha channel of DIB-R's VertexColor renderer: (B,H,W).  Differentiable w.r.t. verts.
     `pixels` (1-D LongTensor of flat pixel indices h*W+w) restricts the evaluation to those pixels and returns
     (B, len(pixels)) - used to check BASELINE-size meshes (F = 16 128 / 32 256) on a pixel subset.
+    `knum` is the number of soft candidates a pixel keeps (DIB-R: 30; the C ABI accepts 1..32).
 
     Back faces (normal.z < 0): the hard pass skips them (`if (direction < 0) continue;` in DIB-R's render kernel); the
     soft pass does NOT (its kernel receives only the 2-D points, the expanded boxes and the coverage index - SURVEY.md
@@ -560,75 +669,17 @@ def soft_silhouette(verts: torch.Tensor, faces: torch.Tensor, rot: torch.Tensor,
     (min over 3 edge-perpendicular distances whose foot lies on the segment, else 4 mult^2, and 3
     vertex distances); at most `knum` faces are recorded; alpha = 1 - prod(1 - prob).
     The selections (coverage, bbox, first-knum, min case, foot test) carry no gradient.
+    A face with a non-finite screen coordinate takes part in neither pass (_sil_faces; DESIGN.md section 2).
     """
-    b, v, _ = verts.shape
-    f = faces.size(0)
-    cam, xy = project_vertices(verts, rot, pos)
+    b = verts.shape[0]
     mult = DIBR_MULTIPLIER
-    # per-face data
-    p0c, p1c, p2c = cam[:, faces[:, 0]], cam[:, faces[:, 1]], cam[:, faces[:, 2]]       # (B,F,3)
-    normal_z = torch.cross(p1c - p0c, p2c - p0c, dim=2)[:, :, 2]                          # (B,F)
-    s = torch.stack([xy[:, faces[:, 0]], xy[:, faces[:, 1]], xy[:, faces[:, 2]]], dim=2) * mult  # (B,F,3,2)
-    bmin = s.min(dim=2)[0]
-    bmax = s.max(dim=2)[0]
-    bmin2 = bmin - DIBR_EXPAND * mult
-    bmax2 = bmax + DIBR_EXPAND * mult
-    # pixel centres
-    wi = torch.arange(width, dtype=torch.float32)
-    hi = torch.arange(height, dtype=torch.float32)
-    x0 = (mult / width) * (2 * wi + 1 - width)            # (W,)
-    y0 = (mult / height) * (height - 2 * hi - 1)          # (H,)
-    X = x0[None, :].expand(height, width).reshape(-1)     # (HW,)
-    Y = y0[:, None].expand(height, width).reshape(-1)
-    if pixels is not None:
-        X, Y = X[pixels], Y[pixels]
+    s, front, live = _sil_faces(verts, faces, rot, pos)
+    X, Y = _sil_pixel_centres(height, width, pixels)
+    Xp, Yp = X[:, None], Y[:, None]                        # (P,1)
     out = torch.zeros(b, X.numel())
-    front = (normal_z >= 0)                                # direction < 0 -> skipped
     for bi in range(b):
-        sb = s[bi]                                         # (F,3,2)
-        ax, ay = sb[:, 0, 0][None], sb[:, 0, 1][None]      # (1,F)
-        bx, by = sb[:, 1, 0][None], sb[:, 1, 1][None]
-        cx, cy = sb[:, 2, 0][None], sb[:, 2, 1][None]
-        Xp, Yp = X[:, None], Y[:, None]                    # (HW,1)
-        with torch.no_grad():
-            in_tight = (Xp >= bmin[bi, :, 0][None]) & (Xp < bmax[bi, :, 0][None]) & \
-                       (Yp >= bmin[bi, :, 1][None]) & (Yp < bmax[bi, :, 1][None])
-            m_, p_, n_, q_ = bx - ax, by - ay, cx - ax, cy - ay
-            s_, t_ = Xp - ax, Yp - ay
-            k1 = s_ * q_ - n_ * t_
-            k2 = m_ * t_ - s_ * p_
-            k3 = m_ * q_ - n_ * p_
-            w1 = k1 / (k3 + DIBR_EPS)
-            w2 = k2 / (k3 + DIBR_EPS)
-            w0 = 1 - w1 - w2
-            inside = in_tight & front[bi][None] & (w0 >= 0) & (w1 >= 0) & (w2 >= 0)
-            covered = inside.any(dim=1)                    # (HW,)
-            in_soft = (Xp >= bmin2[bi, :, 0][None]) & (Xp < bmax2[bi, :, 0][None]) & \
-                      (Yp >= bmin2[bi, :, 1][None]) & (Yp < bmax2[bi, :, 1][None])
-            if soft_cull_backfaces:
-                in_soft = in_soft & front[bi][None]
-            rank = torch.cumsum(in_soft.to(torch.int32), dim=1)
-            use = in_soft & (rank <= DIBR_KNUM) & (~covered)[:, None]
-        # squared distance pixel -> triangle, 6 cases
-        pd = []
-        vx = [ax, bx, cx]
-        vy = [ay, by, cy]
-        for i in range(3):
-            x1, y1, x2, y2 = vx[i], vy[i], vx[(i + 1) % 3], vy[(i + 1) % 3]
-            A = y2 - y1
-            Bc = x1 - x2
-            C = x2 * y1 - x1 * y2
-            up = A * Xp + Bc * Yp + C
-            down = A * A + Bc * Bc
-            with torch.no_grad():
-                x3 = (Bc * Bc * Xp - A * Bc * Yp - A * C) / (down + DIBR_EPS)
-                y3 = (A * A * Yp - A * Bc * Xp - Bc * C) / (down + DIBR_EPS)
-                bad = ((x3 - x1) * (x3 - x2) + (y3 - y1) * (y3 - y2)) > 0
-            perp = up * up / (down + DIBR_EPS)
-            pd.append(torch.where(bad, torch.full_like(perp, 4 * mult * mult), perp))
-        for i in range(3):
-            pd.append((Xp - vx[i]) ** 2 + (Yp - vy[i]) ** 2)
-        pd = torch.stack(pd, dim=2)                         # (HW,F,6)
+        covered, _, use = _sil_select(s[bi], front[bi], live[bi], Xp, Yp, soft_cull_backfaces, knum)
+        pd, _ = _sil_dist2(s[bi], Xp, Yp)                  # (P,F,6)
         with torch.no_grad():
             case = torch.argmin(pd, dim=2, keepdim=True)    # first minimum, like the `>` scan
         d2 = torch.gather(pd, 2, case).squeeze(2)
@@ -639,7 +690,8 @@ def soft_silhouette(verts: torch.Tensor, faces: torch.Tensor, rot: torch.Tensor,
     return out if pixels is not None else out.view(b, height, width)
 
 
-def silhouette_loss(verts, faces, gt, dists, elevs, azims, loss_func: str = "L1", soft_cull_backfaces: bool = False) -> torch.Tensor:
+def silhouette_loss(verts, faces, gt, dists, elevs, azims, loss_func: str = "L1", soft_cull_backfaces: bool = False,
+                    knum: int = DIBR_KNUM) -> torch.Tensor:
     """loss/silhouette.py:13-23 + render/vertex_renderer.py:15-26: per-sample look-at camera,
     soft alpha (B,1,H,W), then L1Loss / MSELoss (mean over B*H*W) vs gt (B,1,H,W)."""
     b = verts.size(0)
@@ -647,7 +699,7 @@ def silhouette_loss(verts, faces, gt, dists, elevs, azims, loss_func: str = "L1"
     cams = [look_at_camera(float(azims[i]), float(elevs[i]), float(dists[i])) for i in range(b)]
     rot = torch.stack([c[0] for c in cams])
     pos = torch.stack([c[1] for c in cams])
-    alpha = soft_silhouette(verts, faces, rot, pos, h, w, soft_cull_backfaces=soft_cull_backfaces)[:, None]
+    alpha = soft_silhouette(verts, faces, rot, pos, h, w, soft_cull_backfaces=soft_cull_backfaces, knum=knum)[:, None]
     if loss_func == "L1":
         return (alpha - gt).abs().mean()
     return ((alpha - gt) ** 2).mean()

@@ -86,18 +86,21 @@ sil_faces_kernel(const float* __restrict__ cam, const float* __restrict__ xy,
   r.cx = __fmul_rn(s2[0], mult); r.cy = __fmul_rn(s2[1], mult);
   r.front = (nz >= 0.0f) ? 1.0f : 0.0f;      // kaolin: `if (direction < 0) continue;`
   r.pad = 0.f;
+  // A face with a non-finite coordinate (a NaN vertex, or one on the camera plane: cam.z = 0) takes part in neither
+  // pass.  fminf / fmaxf drop NaN, so one NaN vertex would still leave a box around the other two: all six coordinates
+  // become NaN, every box test of walk_warp_faces fails, and the face's group box below stays empty.
+  const bool finite = isfinite(r.ax) && isfinite(r.ay) && isfinite(r.bx) && isfinite(r.by) && isfinite(r.cx) && isfinite(r.cy);
+  if (!finite) r.ax = r.ay = r.bx = r.by = r.cx = r.cy = __int_as_float(0x7fffffff);
   rec[(size_t)b * F + f] = r;
   if (normals) {
     float len = sqrtf(nx * nx + ny * ny + nz * nz) + 1e-15f;
     float* n = normals + 3 * ((size_t)b * F + f);
     n[0] = nx / len; n[1] = ny / len; n[2] = nz / len;
   }
-  if (r.front > 0.5f || !cull_soft)
+  if (finite && (r.front > 0.5f || !cull_soft))
     box = make_float4(__fsub_rn(min3(r.ax, r.bx, r.cx), em), __fadd_rn(max3(r.ax, r.bx, r.cx), em),
                       __fsub_rn(min3(r.ay, r.by, r.cy), em), __fadd_rn(max3(r.ay, r.by, r.cy), em));
   }
-  // NaN coordinates must not hide a batch: fminf / fmaxf drop NaN operands, so a NaN box is widened to everything
-  if (!(box.x == box.x) || !(box.y == box.y) || !(box.z == box.z) || !(box.w == box.w)) box = make_float4(-inf, inf, -inf, inf);
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     box.x = fminf(box.x, __shfl_xor_sync(0xffffffffu, box.x, o)); box.y = fmaxf(box.y, __shfl_xor_sync(0xffffffffu, box.y, o));
