@@ -122,26 +122,86 @@ def _image_loss(alpha, silhouettes, kind: str, weight: float):
     return sil * weight
 
 
-def _capture(run, device, warmup: int):
-    """Run `run` `warmup` times on a side stream (caches, function attributes, allocator), then capture one call into a
-    CUDA graph.  Returns (graph, what the captured call returned, our kernel launches in one replay)."""
+def _capture(run, device, warmup: int, warm=None, pool=None):
+    """Run `warm` (default: `run`) `warmup` times on a side stream (caches, function attributes, allocator), then capture
+    one call of `run` into a CUDA graph, in memory pool `pool` when given.  Returns (graph, what the captured call
+    returned, our kernel launches in one replay)."""
     from . import _lib
     side = torch.cuda.Stream(device=device)
     side.wait_stream(torch.cuda.current_stream(device))
     with torch.cuda.stream(side):
         for _ in range(warmup):
-            run()
+            (warm or run)()
     torch.cuda.current_stream(device).wait_stream(side)
     torch.cuda.synchronize(device)
     lib = _lib.load()
     n0 = lib.vpn_launch_count()
     graph = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(graph):
+    with torch.cuda.graph(graph, pool=pool):
         outs = run()
     return graph, outs, int(lib.vpn_launch_count() - n0)
 
 
+class _Captured:
+    """One batch size's graph: the static inputs it reads, its static outputs and its per-term losses."""
+
+    def __init__(self, graph, inputs, outputs, terms, launches):
+        self.graph, self.inputs, self.outputs, self.terms, self.launches = graph, inputs, outputs, terms, launches
+
+
+class _GraphedStep:
+    """What the graphed steps share: one CUDA graph per batch size.  The graph of the batch size `batch` of the example
+    tensors is captured at construction.  A smaller batch b (the short last batch of an epoch, or a smaller data-parallel
+    shard) replays a graph captured the first time b is seen and cached by b; it reads the leading b rows of the static
+    input buffers.  The smaller graphs capture into the full-size graph's memory pool: one step object's graphs are only
+    replayed one after another on one stream, so they may share memory.  Every output is a static buffer of the graph
+    that produced it, overwritten by the next call of any size.
+
+    Subclasses implement _static_inputs(b) -> dict, the leading b rows of their static input buffers (the gradient
+    leaves made leaves of their own), and _run(b, inputs, collective) -> (loss, *grads, terms dict), the step of batch b
+    on them; `collective` says whether to call after_backward."""
+
+    def _init_graphs(self, batch: int, device, warmup: int):
+        self.batch, self._device, self._warmup = batch, device, warmup
+        self._graphs: Dict[int, _Captured] = {}
+        full = self._graph_for(batch)
+        self.graph, self.launches_per_step, self.terms = full.graph, full.launches, full.terms
+        return full.outputs
+
+    def _rows(self, x, b: int):
+        """The leading b rows of a static input (a tensor, a tuple of them, or None); the input itself at full size."""
+        if x is None or b == self.batch:
+            return x
+        if isinstance(x, tuple):
+            return tuple(c[:b] for c in x)
+        return x[:b]
+
+    def _graph_for(self, b: int) -> _Captured:
+        """The graph of batch b, captured on first use.  b > batch raises AssertionError before any copy or launch."""
+        assert b <= self.batch, f"batch of {b} samples: the step was captured for at most {self.batch}"
+        hit = self._graphs.get(b)
+        if hit is not None:
+            return hit
+        inputs = self._static_inputs(b)
+        run = lambda: self._run(b, inputs, collective=True)
+        # a lazy capture's eager warm-up steps leave out after_backward: under data parallelism the ranks' shards may
+        # differ in size, so one rank may capture while the others replay, and each rank must run exactly one collective
+        # per step.  The captured graph contains it, as the full-size one does.
+        warm = None if not self._graphs else (lambda: self._run(b, inputs, collective=False))
+        pool = None if not self._graphs else self._graphs[self.batch].graph.pool()
+        graph, outs, launches = _capture(run, self._device, self._warmup, warm=warm, pool=pool)
+        hit = self._graphs[b] = _Captured(graph, inputs, outs[:-1], outs[-1], launches)
+        return hit
+
+    def _replay(self, g: _Captured):
+        g.graph.replay()
+        self.terms = g.terms
+        return g.outputs
+
+
 class PrimitiveLoss(_LossStep):
+    TERMS = ("view_cd", "obj_cd", "vp_div", "emd", "sil")        # the output's weighted terms, in the order they are summed
+
     def __init__(self, config: Optional[PrimitiveLossConfig] = None):
         self.cfg = config or PrimitiveLossConfig()
         assert self.cfg.kind in ("sphere", "cuboid", "mixed")
@@ -278,7 +338,7 @@ class PrimitiveLoss(_LossStep):
         return _image_loss(alpha, silhouettes, cfg.silhouette_loss, cfg.l_sil), alpha
 
 
-class GraphedPrimitiveLoss:
+class GraphedPrimitiveLoss(_GraphedStep):
     """The same step - draw uniforms, forward, backward to (v, q, t) - captured once into a CUDA graph and replayed.
 
     The step is ~20 of our launches plus torch's bookkeeping kernels; at small batch sizes (BASELINE config 1: B = 1) and
@@ -288,14 +348,22 @@ class GraphedPrimitiveLoss:
 
         g = GraphedPrimitiveLoss(cfg, v, q, t, targets, silhouettes)      # example tensors give the shapes
         loss, gv, gq, gt = g(v, q, t, targets, silhouettes)               # static output buffers, overwritten by the next call
-    """
+        g.terms                                                           # {"view_cd": ..., "vp_div": ..., ...} of that call
+
+    `terms` holds the weighted terms of the last call, as PrimitiveLoss returns them (only those with a non-zero weight,
+    each multiplied by its weight): 0-d tensors the captured forward writes, so reading them adds no kernel to the
+    replay; like the other outputs they are overwritten by the next call.  A batch smaller than the example batch (the
+    epoch's short last batch) replays a graph of its own size, captured on first use (_GraphedStep)."""
 
     def __init__(self, config: PrimitiveLossConfig, v, q, t, targets, silhouettes=None, n_samples: int = 0, warmup: int = 3,
-                 canonical_points=None, cameras=None, after_backward=None):
+                 canonical_points=None, cameras=None, after_backward=None, sil_cameras=None):
         """after_backward: optional callable queued on the step's stream after the backward pass and captured with it -
         e.g. GradientAllReduce.launch(inline=True) when the all-reduce is our own self-synchronising kernel, so that no
         host launch sits between the step's tail and the collective.  It also runs in each of the `warmup` eager steps
-        (every rank makes the same number of calls)."""
+        here (every rank makes the same number of calls), but not in the warm-up steps of a smaller batch's lazy capture:
+        a rank may capture that graph while the others replay theirs, and each captured graph runs it exactly once.
+        sil_cameras: (dists, elevs, azims) (B,) to render the silhouette from, as PrimitiveLoss(..., sil_cameras=)
+        (train.py with IS_VIEW_CENTER = False); without them the view-centred camera is used."""
         self.cfg = config
         self.step = PrimitiveLoss(config)
         dev = v.device
@@ -307,54 +375,73 @@ class GraphedPrimitiveLoss:
         # canonical-frame Chamfer of train.py:152-163: targets in the object frame + (dists, elevs, azims, angles)
         self.canonical = None if canonical_points is None else canonical_points.detach().clone()
         self.cameras = None if cameras is None else tuple(c.detach().clone() for c in cameras)
+        self.sil_cameras = None if sil_cameras is None else tuple(c.detach().clone() for c in sil_cameras)
+        self.n_samples = n_samples
+        self._after_backward = after_backward
         b, k = q.shape[:2]
-        if config.vertex_chamfer:
-            self.ushape = None
-        elif config.kind == "mixed":
-            kc = config.n_cuboids
-            assert kc <= k, f"n_cuboids = {kc} exceeds the K = {k} primitives"
-            self.ushape = ((b, kc, n_samples, 3), (b, k - kc, n_samples, 2))      # u_cuboid, then u_sphere
-        else:
-            self.ushape = (b, k, n_samples, 2 if config.kind == "sphere" else 3)
+        if config.kind == "mixed":
+            assert config.n_cuboids <= k, f"n_cuboids = {config.n_cuboids} exceeds the K = {k} primitives"
+        self.ushape = self._ushape(b)
         assert config.vertex_chamfer or n_samples > 0, "n_samples (points per primitive) is required unless vertex_chamfer"
-
-        def draw():
-            if self.ushape is None:
-                return None
-            if config.kind == "mixed":
-                return tuple(torch.rand(shape, device=dev) for shape in self.ushape)
-            return torch.rand(self.ushape, device=dev)
 
         # seeds autograd.grad of the total: made once, outside the capture, so a replay has no fill kernel for it.  The
         # graph reads it at every replay, so the object keeps it alive.
         self._one = torch.ones((), device=dev)
+        self.loss, self.gv, self.gq, self.gt = self._init_graphs(b, dev, warmup)
 
-        def run():
-            u = draw()      # drawn on the device, as the reference does
-            cams = self.cameras or (None, None, None, None)
-            out = self.step(self.v, self.q, self.t, u, self.targets, silhouettes=self.sil, canonical_points=self.canonical,
-                            dists=cams[0], elevs=cams[1], azims=cams[2], angles=cams[3])
-            gv, gq, gt = torch.autograd.grad(out["total"], (self.v, self.q, self.t), grad_outputs=self._one)
-            if after_backward is not None:
-                after_backward()
-            return out["total"], gv, gq, gt
+    def _ushape(self, b: int):
+        """Shape of the uniforms of b samples (a pair under 'mixed'; None on the vertex path)."""
+        cfg, k, n = self.cfg, self.q.shape[1], self.n_samples
+        if cfg.vertex_chamfer:
+            return None
+        if cfg.kind == "mixed":
+            kc = cfg.n_cuboids
+            return (b, kc, n, 3), (b, k - kc, n, 2)                  # u_cuboid, then u_sphere
+        return b, k, n, 2 if cfg.kind == "sphere" else 3
 
-        self.graph, (self.loss, self.gv, self.gq, self.gt), self.launches_per_step = _capture(run, dev, warmup)
+    def _static_inputs(self, b: int):
+        if b == self.batch:
+            leaves = (self.v, self.q, self.t)
+        else:
+            leaves = tuple(x.detach()[:b].requires_grad_() for x in (self.v, self.q, self.t))
+        return dict(zip(("v", "q", "t"), leaves), targets=self._rows(self.targets, b), sil=self._rows(self.sil, b),
+                    canonical=self._rows(self.canonical, b), cameras=self._rows(self.cameras, b),
+                    sil_cameras=self._rows(self.sil_cameras, b))
 
-    def __call__(self, v, q, t, targets, silhouettes=None, canonical_points=None, cameras=None):
-        if self.canonical is not None and canonical_points is not None:
-            self.canonical.copy_(canonical_points, non_blocking=True)
-        if self.cameras is not None and cameras is not None:
-            for dst, src in zip(self.cameras, cameras):
-                dst.copy_(src, non_blocking=True)
-        self.v.data.copy_(v, non_blocking=True)
-        self.q.data.copy_(q, non_blocking=True)
-        self.t.data.copy_(t, non_blocking=True)
-        self.targets.copy_(targets, non_blocking=True)
-        if self.sil is not None and silhouettes is not None:
-            self.sil.copy_(silhouettes, non_blocking=True)
-        self.graph.replay()
-        return self.loss, self.gv, self.gq, self.gt
+    def _run(self, b: int, x, collective: bool):
+        ushape = self._ushape(b)
+        dev = self.v.device
+        if ushape is None:
+            u = None
+        elif self.cfg.kind == "mixed":
+            u = tuple(torch.rand(shape, device=dev) for shape in ushape)
+        else:
+            u = torch.rand(ushape, device=dev)                       # drawn on the device, as the reference does
+        cams = x["cameras"] or (None, None, None, None)
+        out = self.step(x["v"], x["q"], x["t"], u, x["targets"], silhouettes=x["sil"], canonical_points=x["canonical"],
+                        dists=cams[0], elevs=cams[1], azims=cams[2], angles=cams[3], sil_cameras=x["sil_cameras"])
+        gv, gq, gt = torch.autograd.grad(out["total"], (x["v"], x["q"], x["t"]), grad_outputs=self._one)
+        if collective and self._after_backward is not None:
+            self._after_backward()
+        return out["total"], gv, gq, gt, {k: out[k] for k in PrimitiveLoss.TERMS if k in out}
+
+    def __call__(self, v, q, t, targets, silhouettes=None, canonical_points=None, cameras=None, sil_cameras=None):
+        """A batch of b <= B samples (B: the example batch); b < B replays the graph of b, captured on first use."""
+        g = self._graph_for(q.shape[0])
+        x = g.inputs
+        if x["canonical"] is not None and canonical_points is not None:
+            x["canonical"].copy_(canonical_points, non_blocking=True)
+        for static, given in ((x["cameras"], cameras), (x["sil_cameras"], sil_cameras)):
+            if static is not None and given is not None:
+                for dst, src in zip(static, given):
+                    dst.copy_(src, non_blocking=True)
+        x["v"].data.copy_(v, non_blocking=True)
+        x["q"].data.copy_(q, non_blocking=True)
+        x["t"].data.copy_(t, non_blocking=True)
+        x["targets"].copy_(targets, non_blocking=True)
+        if x["sil"] is not None and silhouettes is not None:
+            x["sil"].copy_(silhouettes, non_blocking=True)
+        return self._replay(g)
 
 
 @dataclass
@@ -388,6 +475,8 @@ class MeshLoss(_LossStep):
 
     train_sphere.py passes verts = template + offsets (the offsets' gradient is the vertices'); train_gcn.py passes the
     network's vertices.  The branches are placed on streams as in PrimitiveLoss."""
+
+    TERMS = ("cd", "emd", "sil")                                   # the output's weighted terms, in the order they are summed
 
     def __init__(self, config: Optional[MeshLossConfig] = None):
         self.cfg = config or MeshLossConfig()
@@ -460,15 +549,17 @@ class MeshLoss(_LossStep):
         return _image_loss(alpha, silhouettes, cfg.silhouette_loss, cfg.l_sil), alpha
 
 
-class GraphedMeshLoss:
+class GraphedMeshLoss(_GraphedStep):
     """MeshLoss - draw the uniforms, forward, backward to the vertices - captured once into a CUDA graph and replayed,
     as GraphedPrimitiveLoss does for the primitive step.  The topology is fixed at construction; vertices, targets and
     silhouettes are copied into static buffers, results are read from static buffers.
 
         g = GraphedMeshLoss(cfg, verts, faces, targets, silhouettes)   # example tensors give the shapes
         loss, grad_verts = g(verts, targets, silhouettes)             # overwritten by the next call
+        g.terms                                                       # {"cd": ..., "sil": ..., "emd": ...} of that call
         offsets.backward(grad_verts)                                  # train_sphere.py: verts = template + offsets
-    """
+
+    `terms` and batches smaller than the example batch work as in GraphedPrimitiveLoss."""
 
     def __init__(self, config: MeshLossConfig, verts, faces, targets, silhouettes=None, warmup: int = 3):
         self.cfg = config
@@ -481,23 +572,29 @@ class GraphedMeshLoss:
 
         self._one = torch.ones((), device=dev)       # as in GraphedPrimitiveLoss
 
-        def run():
-            out = self.step(self.verts, self.faces, self.targets, silhouettes=self.sil)
-            (gv,) = torch.autograd.grad(out["total"], (self.verts,), grad_outputs=self._one)
-            return out["total"], gv
-
         # the sampler's backward reads the cached vertex CSR of these faces: build it before the capture and keep it
         # alive as long as the graph
         self._adjacency = ops.mesh_adjacency(self.faces, verts.size(1)) if config.n_samples and verts.is_cuda else None
-        self.graph, (self.loss, self.gv), self.launches_per_step = _capture(run, dev, warmup)
+        self.loss, self.gv = self._init_graphs(verts.size(0), dev, warmup)
+
+    def _static_inputs(self, b: int):
+        verts = self.verts if b == self.batch else self.verts.detach()[:b].requires_grad_()
+        return dict(verts=verts, targets=self._rows(self.targets, b), sil=self._rows(self.sil, b))
+
+    def _run(self, b: int, x, collective: bool):
+        out = self.step(x["verts"], self.faces, x["targets"], silhouettes=x["sil"])
+        (gv,) = torch.autograd.grad(out["total"], (x["verts"],), grad_outputs=self._one)
+        return out["total"], gv, {k: out[k] for k in MeshLoss.TERMS if k in out}
 
     def __call__(self, verts, targets, silhouettes=None):
-        self.verts.data.copy_(verts, non_blocking=True)
-        self.targets.copy_(targets, non_blocking=True)
-        if self.sil is not None and silhouettes is not None:
-            self.sil.copy_(silhouettes, non_blocking=True)
-        self.graph.replay()
-        return self.loss, self.gv
+        """A batch of b <= B meshes (B: the example batch); b < B replays the graph of b, captured on first use."""
+        g = self._graph_for(verts.size(0))
+        x = g.inputs
+        x["verts"].data.copy_(verts, non_blocking=True)
+        x["targets"].copy_(targets, non_blocking=True)
+        if x["sil"] is not None and silhouettes is not None:
+            x["sil"].copy_(silhouettes, non_blocking=True)
+        return self._replay(g)
 
 
 class HostPipeline:
@@ -516,7 +613,12 @@ class HostPipeline:
     batch is queued as soon as it is submitted (behind the previous one), so the device never waits for the host between
     steps, and the host synchronises once per step, on the oldest outstanding result.  `pre_step` (optional) is queued
     on the compute stream before every step (the bench's L2 flush).  On a CPU device everything runs synchronously (the
-    ordering logic is the same; used by the tests)."""
+    ordering logic is the same; used by the tests).
+
+    A batch whose tensors have fewer rows than the example batch's (an epoch's short last batch) is staged into the
+    leading rows of the slot, and the step gets views of those rows.  Pinned host result buffers are allocated per
+    output shape, the first time a slot sees it.  A step that also wants a graphed step's per-term losses returns them
+    with its results, e.g. lambda s: (*g(s["v"], ...), *g.terms.values())."""
 
     def __init__(self, step, example_batch: Dict[str, Optional[torch.Tensor]], device, pre_step=None):
         self.step, self.pre_step = step, pre_step
@@ -525,6 +627,7 @@ class HostPipeline:
         self.staging = [{k: (None if v is None else torch.empty(v.shape, dtype=v.dtype, device=self.device))
                          for k, v in example_batch.items()} for _ in range(2)]
         self.host_out: list = [None, None]
+        self._host_bufs: list = [{}, {}]                             # per slot: output shapes -> pinned host buffers
         self.submitted = 0
         self.returned = 0
         if self.cuda:
@@ -541,6 +644,11 @@ class HostPipeline:
         assert self.submitted - self.returned < 2, "two batches are already in flight: call result() first"
         slot = self.submitted % 2
         st = self.staging[slot]
+        for k, v in batch.items():
+            if v is not None:
+                assert v.shape[0] <= st[k].shape[0], f"batch['{k}'] has {v.shape[0]} rows, the example batch {st[k].shape[0]}"
+        if any(v is not None and v.shape[0] < st[k].shape[0] for k, v in batch.items()):
+            st = {k: (x if x is None or batch.get(k) is None else x[:batch[k].shape[0]]) for k, x in st.items()}
         if self.cuda:
             cur = torch.cuda.current_stream(self.device)
             with torch.cuda.stream(self.copy_stream):
@@ -566,8 +674,10 @@ class HostPipeline:
         outs = self.step(st)
         if self.cuda:
             self.free[slot].record(cur)
-        if self.host_out[slot] is None:
-            self.host_out[slot] = [torch.empty(o.shape, dtype=o.dtype, pin_memory=self.cuda) for o in outs]
+        key = tuple((tuple(o.shape), o.dtype) for o in outs)
+        if key not in self._host_bufs[slot]:
+            self._host_bufs[slot][key] = [torch.empty(o.shape, dtype=o.dtype, pin_memory=self.cuda) for o in outs]
+        self.host_out[slot] = self._host_bufs[slot][key]
         for h, o in zip(self.host_out[slot], outs):
             h.copy_(o.detach(), non_blocking=True)
         if self.cuda:
